@@ -8,7 +8,7 @@ Workload: BASELINE config 3, Oberrhein feeder (N=70 buses, E=69 closed branches)
 synthetic scenarios from the deterministic generator (dss2.synth; the reference's Oberrhein scenario pickles are missing
 from its repository), random-init weights.  Weak scaling: every rank owns its own shard and batch.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Prints ONE JSON line on rank 0 (see the task's contract): value = device-resident throughput, e2e = through the host-buffer
 API (pinned host scenarios -> H2D -> step -> D2H loss) inside the timed region, roofline = the dominant kernel (TAG-layer
@@ -80,7 +80,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch eagerly instead of replaying a CUDA graph")
     ap.add_argument("--same-shards", action="store_true", help="every rank uses rank 0's scenarios and ids (multi-GPU == single-GPU check)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0), so that two builds "
+                         "can be compared output for output on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.batch is None:
         args.batch = CONFIGS[args.config][1]
     if args.scenarios is None:
@@ -185,6 +192,41 @@ def run_reference(args):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
+# --dump-outputs
+# ---------------------------------------------------------------------------------------------------------------------
+DUMP_BUDGET = 60 << 20   # bytes of array data in all: with the .npy headers the dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every tensor of `arrays` as out_dir/<name>.npy, float64 tensors as float64 and all others as float32.  Should the arrays
+    exceed DUMP_BUDGET together, each one larger than an even share of it keeps a seeded random sample of its rows in their original
+    order (of its entries, flattened, when one row alone exceeds the share): the same rows in every run with the same shapes, so dumps
+    of two builds still compare entry for entry."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    share = DUMP_BUDGET // len(host)
+    sample = sum(a.nbytes for a in host.values()) > DUMP_BUDGET
+    for name, a in host.items():
+        if sample and a.nbytes > share:
+            if a.nbytes // a.shape[0] > share:
+                a = a.reshape(-1)
+            rows = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def named_parameters_flat(params):
+    """{name: tensor} -> one vector, concatenated in the order of the sorted names: independent of how a build lays the parameters
+    out in its flat buffer."""
+    import torch
+    return torch.cat([params[k].detach().reshape(-1) for k in sorted(params)])
+
+
+# ---------------------------------------------------------------------------------------------------------------------
 # clocks
 # ---------------------------------------------------------------------------------------------------------------------
 class ClockSampler(threading.Thread):
@@ -241,13 +283,16 @@ def run_eager(args, dev, rank, world, local, K, W):
     opt = torch.optim.Adamax(model.parameters(), lr=3e-3)
     stats = [t.to(dev) for t in (store.x_mean, store.x_std, store.edge_mean, store.edge_std)]
     x, ea, ei = batch.x, batch.edge_attr, batch.edge_index
+    last = {}      # what the latest step handed its caller (for --dump-outputs)
 
     def step():
         if args.mode == "infer":                                   # dss2_run.py:177-194
             with torch.no_grad():
                 out = model(x[:, :8], ei, ea[:, :6])
                 est = torch.cat([out[:, 0:1] * stats[1][:1] + stats[0][:1], out[:, 1:] * (1. - x[:, 9:10])], 1)
-                return d3.get_pflow(est, ei, node_param=x[:, 8:], edge_param=ea[:, 6:])[0].sum()
+                pflow = d3.get_pflow(est, ei, node_param=x[:, 8:], edge_param=ea[:, 6:])
+                last.update(output=out, pflow=pflow)
+                return pflow[0].sum()
         opt.zero_grad(set_to_none=True)                            # dss2_run.py:137-143
         out = model(x[:, :8], ei, ea[:, :6])
         loss = d3.gsp_wls_edge(input=x[:, :8], edge_input=ea[:, :6], output=out, x_mean=stats[0], x_std=stats[1], edge_mean=stats[2],
@@ -274,6 +319,9 @@ def run_eager(args, dev, rank, world, local, K, W):
     sampler.join()
     ms = a.elapsed_time(b)
     launches = _lib.launch_count() - n0
+    if args.dump_outputs:   # inference (training runs through GraphedTrainer in main); pflow columns: loading_lines, loading_trafo,
+        # P_from, Q_from, P_to, Q_to, I_from, I_to
+        dump_outputs(args.dump_outputs, {"output": last["output"], "pflow": torch.stack(last["pflow"], dim=1)})
     # end to end: the batch's features come from pinned host memory every step, the scalar result goes back
     hx, hea = x.cpu().pin_memory(), ea.cpu().pin_memory()
     hres = torch.zeros(1).pin_memory()
@@ -380,6 +428,9 @@ def main():
     sampler.join()
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     loss_end = float(trainer.loss.item())
+    if args.dump_outputs and rank == 0:   # before the kernel timings below reuse the trainer's buffers
+        dump_outputs(args.dump_outputs, {"loss": trainer.loss, "loss_per_step": loss_hist,
+                                         "parameters": named_parameters_flat(trainer.state_dict())})
     value = world * B * K / (ms_total / 1e3)
     # data-parallel sanity, outside the timed region: every replica must hold bit-identical parameters after the K steps (same
     # all-reduced gradient, same update), and with --same-shards the loss trajectory must be the one a single GPU produces

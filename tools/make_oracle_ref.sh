@@ -3,13 +3,13 @@
 # git-ignored oracle/_ref/ (never committed; it travels to the GPU box with the gpurun snapshot like a built .so).  bench.py's
 # `--impl reference` arm and the dss2_run.py exec test run these files over oracle/pyg_shim (torch_geometric is not installable
 # here).  Nothing in the product package reads oracle/_ref/.
-#   usage: tools/make_oracle_ref.sh [reference_root]        (default /root/reference)
+#   usage: tools/make_oracle_ref.sh [reference_root]        (default: $DSS2_REFERENCE)
 set -e
-REF="${1:-/root/reference}"
+REF="${1:-${DSS2_REFERENCE:-}}"
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"
 DST="$ROOT/oracle/_ref"
-if [ ! -f "$REF/networks.py" ]; then
-  echo "make_oracle_ref: $REF/networks.py not found (no reference checkout on this machine); keeping whatever is in $DST" >&2
+if [ -z "$REF" ] || [ ! -f "$REF/networks.py" ]; then
+  echo "make_oracle_ref: no reference checkout (argument or DSS2_REFERENCE: '$REF'); keeping whatever is in $DST" >&2
   exit 0
 fi
 mkdir -p "$DST"
