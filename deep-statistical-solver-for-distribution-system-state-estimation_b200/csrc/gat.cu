@@ -32,6 +32,47 @@ constexpr int GAT_SLOTS = 8;
 __constant__ GatW c_gat[GAT_SLOTS];
 __device__ GatW g_gat_stage[GAT_SLOTS];
 
+// Attention dropout (GATv2Conv / FAConv `dropout`, applied to the normalised coefficients in training mode).  The keep bit of an
+// attention coefficient is a pure function of (seed, step, layer_uid, head, edge key): edge key = one-way edge id for a real edge (the
+// destination's entry and the source's reversed entry see the same bit), Et + i for the loop appended at bus i.  Every site that
+// visits the coefficient (forward, statistics pass, both backward branches) re-draws the same bit; nothing is stored.
+struct AttnDropArgs {
+  int mode;             // 1 philox (seed / step from rng[0..1] on the device), 2 caller mask (uint8 [Et + Nt], 1 = keep)
+  float scale;          // 1 / (1 - p)
+  uint32_t keep_thr;    // philox: keep iff draw < keep_thr
+  uint32_t layer_uid, head;
+  const uint64_t* rng;
+  const uint8_t* mask;
+  int64_t num_edges;    // Et: first edge key of the appended loops
+};
+// third counter word: every TAG dropout draw puts a value below 32 there, so this domain tag keeps the two streams disjoint
+constexpr uint32_t ATTN_DROP_DOMAIN = 0xA7700000u;
+struct AttnKey {
+  uint2 key;
+  uint32_t step_lo;
+};
+__device__ __forceinline__ AttnKey attn_key(const AttnDropArgs& d) {
+  AttnKey k = {make_uint2(0u, 0u), 0u};
+  if (d.mode == 1) {
+    const uint64_t seed = d.rng[0], step = d.rng[1];
+    k.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32) ^ (d.layer_uid * 0x9E3779B9u) ^ (uint32_t)(step >> 32));
+    k.step_lo = (uint32_t)step;
+  }
+  return k;
+}
+__device__ __forceinline__ bool attn_keep(const AttnDropArgs& d, const AttnKey& k, uint64_t e) {
+  if (d.mode == 2) return d.mask[e] != 0;
+  const uint4 q = philox4x32_10(make_uint4((uint32_t)e, (uint32_t)(e >> 32), ATTN_DROP_DOMAIN | d.head, k.step_lo), k.key);
+  return q.x < d.keep_thr;
+}
+// d_k = mask_k / (1 - p): the factor the coefficient of edge key e is multiplied with
+__device__ __forceinline__ float attn_factor(const AttnDropArgs& d, const AttnKey& k, uint64_t e) { return attn_keep(d, k, e) ? d.scale : 0.0f; }
+
+__global__ void k_attn_drop_mask(AttnDropArgs d, int64_t n, uint8_t* out) {
+  const AttnKey k = attn_key(d);
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) out[e] = attn_keep(d, k, e) ? 1 : 0;
+}
+
 struct GatArgs {
   dss2_graph_t g;
   const float* x;
@@ -51,6 +92,7 @@ struct GatArgs {
   float* partials;     // k_gat_bwd: the lin_edge.w block of the partial row
   int64_t partial_stride;
   int64_t off_att, off_bias;   // k_gat_bwd: att and bias blocks relative to `partials`
+  AttnDropArgs drop;           // read by the DROP = true kernels only
 };
 
 __device__ __forceinline__ void load_weights(GatW& w, const GatArgs& a) {
@@ -120,12 +162,13 @@ __device__ __forceinline__ float edge_score(const GatW& w, const float (&s)[GC],
 
 // Per-destination softmax statistics of bus i: max score m, denominator den (incl. PyG's 1e-16), un-normalised weighted sum acc of
 // x_l over the in-edges and the loop, mean in-attribute abar.  `G` (optional) additionally gives t = sum_k alpha_k (G . x_l[k]).
+// DROP: acc and t weight edge k with alpha_k d_k (the denominator is the softmax's, before the dropout).
 struct DstStats {
   float m, den, t;
 };
-template <bool WITH_T>
+template <bool WITH_T, bool DROP = false>
 __device__ __forceinline__ DstStats dst_pass(const GatArgs& a, const GatW& w, int64_t i, const float (&xr)[GC], const float (&xl_i)[GC],
-                                             float (&abar)[GFE], float (&acc)[GC], const float (&G)[GC]) {
+                                             float (&abar)[GFE], float (&acc)[GC], const float (&G)[GC], const AttnKey& dk = AttnKey{}) {
   const dss2_graph_t& g = a.g;
   const int beg = g.rowptr[i], end = g.rowptr[i + 1];
   float m = -INFINITY;
@@ -172,24 +215,28 @@ __device__ __forceinline__ DstStats dst_pass(const GatArgs& a, const GatW& w, in
     edge_pre(w, xr, xl, at, s);
     const float ex = expf(edge_score(w, s, a.slope_att) - m);
     den += ex;
+    float exd = ex;
+    if constexpr (DROP) exd = ex * attn_factor(a.drop, dk, id);
     float dot = 0.0f;
 #pragma unroll
     for (int c = 0; c < GC; ++c) {
-      acc[c] = fmaf(ex, xl[c], acc[c]);
+      acc[c] = fmaf(exd, xl[c], acc[c]);
       if (WITH_T) dot = fmaf(G[c], xl[c], dot);
     }
-    if (WITH_T) t = fmaf(ex, dot, t);
+    if (WITH_T) t = fmaf(exd, dot, t);
   }
   if (a.loops) {
     const float ex = expf(sc_loop - m);
     den += ex;
+    float exd = ex;
+    if constexpr (DROP) exd = ex * attn_factor(a.drop, dk, (uint64_t)a.drop.num_edges + (uint64_t)i);
     float dot = 0.0f;
 #pragma unroll
     for (int c = 0; c < GC; ++c) {
-      acc[c] = fmaf(ex, xl_i[c], acc[c]);
+      acc[c] = fmaf(exd, xl_i[c], acc[c]);
       if (WITH_T) dot = fmaf(G[c], xl_i[c], dot);
     }
-    if (WITH_T) t = fmaf(ex, dot, t);
+    if (WITH_T) t = fmaf(exd, dot, t);
   }
   den += 1e-16f;   // a bus without in-edges and without loop: acc = 0, den = 1e-16 -> out = bias, like PyG's empty softmax segment
   DstStats r;
@@ -199,17 +246,19 @@ __device__ __forceinline__ DstStats dst_pass(const GatArgs& a, const GatW& w, in
   return r;
 }
 
-template <int SLOT>
+template <int SLOT, bool DROP>
 __global__ void __launch_bounds__(GAT_THREADS) k_gat_fwd(GatArgs a) {
   __shared__ GatW w_sh;
   const GatW& w = gat_weights<SLOT>(w_sh, a);
   const float zero[GC] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  AttnKey dk = {};
+  if constexpr (DROP) dk = attn_key(a.drop);
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < a.g.num_nodes; i += (int64_t)gridDim.x * blockDim.x) {
     float xi[GC], xr[GC], xl[GC], abar[GFE], acc[GC];
     load_x(a, i, xi);
     lin8(w.wr, w.br, xi, xr);
     lin8(w.wl, w.bl, xi, xl);
-    const DstStats st = dst_pass<false>(a, w, i, xr, xl, abar, acc, zero);
+    const DstStats st = dst_pass<false, DROP>(a, w, i, xr, xl, abar, acc, zero, dk);
     float out[GC];
 #pragma unroll
     for (int c = 0; c < GC; ++c) {
@@ -223,10 +272,12 @@ __global__ void __launch_bounds__(GAT_THREADS) k_gat_fwd(GatArgs a) {
 }
 
 // backward pass A: per bus g = grad_y * gate, x_r, softmax statistics (m, den, t)
-template <int SLOT>
+template <int SLOT, bool DROP>
 __global__ void __launch_bounds__(GAT_THREADS) k_gat_bwd_stats(GatArgs a) {
   __shared__ GatW w_sh;
   const GatW& w = gat_weights<SLOT>(w_sh, a);
+  AttnKey dk = {};
+  if constexpr (DROP) dk = attn_key(a.drop);
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < a.g.num_nodes; i += (int64_t)gridDim.x * blockDim.x) {
     float xi[GC], xr[GC], xl[GC], abar[GFE], acc[GC], G[GC];
     load_x(a, i, xi);
@@ -238,7 +289,7 @@ __global__ void __launch_bounds__(GAT_THREADS) k_gat_bwd_stats(GatArgs a) {
       const float gate = a.act == 2 ? 1.0f - yv * yv : ((a.act == 1 && !(yv > 0.0f)) ? a.slope_act : 1.0f);
       G[c] = a.gy[i * GC + c] * gate;
     }
-    const DstStats st = dst_pass<true>(a, w, i, xr, xl, abar, acc, G);
+    const DstStats st = dst_pass<true, DROP>(a, w, i, xr, xl, abar, acc, G, dk);
     float* o = a.ws + i * GAT_NODE_WS;
     o[0] = st.m;
     o[1] = st.den;
@@ -251,31 +302,40 @@ __global__ void __launch_bounds__(GAT_THREADS) k_gat_bwd_stats(GatArgs a) {
   }
 }
 
-// adjoint of one edge (j -> i) given the destination's statistics: returns alpha, fills ds = d loss / d s, adds to d att
+// adjoint of one edge (j -> i) given the destination's statistics: returns alpha, fills ds = d loss / d s, adds to d att.
+// DROP (d = the edge's dropout factor): returns alpha d, the weight of x_l[j] in out[i]; d score = alpha (d (G_i . x_l[j]) - t_i).
+template <bool DROP = false>
 __device__ __forceinline__ float edge_adjoint(const GatArgs& a, const GatW& w, const float (&s)[GC], float m, float den, float t,
-                                              const float (&Gi)[GC], const float (&xl_j)[GC], float (&ds)[GC], float* datt) {
+                                              const float (&Gi)[GC], const float (&xl_j)[GC], float (&ds)[GC], float* datt, float d = 1.0f) {
   const float alpha = expf(edge_score(w, s, a.slope_att) - m) / den;
   float dal = 0.0f;
 #pragma unroll
   for (int c = 0; c < GC; ++c) dal = fmaf(Gi[c], xl_j[c], dal);
-  const float dsc = alpha * (dal - t);
+  float dsc;
+  // d * dal rounded on its own (no fused multiply-add), as t's terms were: a segment of one kept coefficient (a bus with one in-edge
+  // and no loop) then gets exactly t = d dal and d score = 0, like the softmax adjoint it stands for
+  if constexpr (DROP) dsc = alpha * (__fmul_rn(d, dal) - t);
+  else dsc = alpha * (dal - t);
 #pragma unroll
   for (int c = 0; c < GC; ++c) {
     const bool pos = s[c] > 0.0f;
     ds[c] = dsc * w.att[c] * (pos ? 1.0f : a.slope_att);
     if (datt) datt[c] = fmaf(dsc, pos ? s[c] : s[c] * a.slope_att, datt[c]);
   }
+  if constexpr (DROP) return alpha * d;
   return alpha;
 }
 
 // backward pass B: thread = bus n.  As destination it owns d x_r[n], d W_e, d att of its in-edges and loop; as source it gathers d x_l[n]
 // from its out-edges.  partial layout per CTA: [W_e 8 x fe | att 8 | bias 8] at the offsets the host passes via partials pointer.
-template <int SLOT>
+template <int SLOT, bool DROP>
 __global__ void __launch_bounds__(GAT_BWD_THREADS) k_gat_bwd(GatArgs a) {
   __shared__ GatW w_sh;
   __shared__ float red[GAT_BWD_THREADS / 32][GC * GFE + 2 * GC];
   const GatW& w = gat_weights<SLOT>(w_sh, a);
   const dss2_graph_t& g = a.g;
+  AttnKey dk = {};
+  if constexpr (DROP) dk = attn_key(a.drop);
   float dWe[GC * GFE], datt[GC], dbias[GC];
 #pragma unroll
   for (int i = 0; i < GC * GFE; ++i) dWe[i] = 0.0f;
@@ -315,7 +375,9 @@ __global__ void __launch_bounds__(GAT_BWD_THREADS) k_gat_bwd(GatArgs a) {
         for (int f = 0; f < GFE; ++f) abar[f] += at[f];
         ++cnt;
         edge_pre(w, xr_n, xl_o, at, s);
-        edge_adjoint(a, w, s, m_n, den_n, t_n, Gn, xl_o, ds, datt);
+        float d = 1.0f;
+        if constexpr (DROP) d = attn_factor(a.drop, dk, id);
+        edge_adjoint<DROP>(a, w, s, m_n, den_n, t_n, Gn, xl_o, ds, datt, d);
 #pragma unroll
         for (int c = 0; c < GC; ++c) {
           dxr[c] += ds[c];
@@ -331,7 +393,9 @@ __global__ void __launch_bounds__(GAT_BWD_THREADS) k_gat_bwd(GatArgs a) {
           xr_o[c] = so[12 + c];
         }
         edge_pre(w, xr_o, xl_n, at, s);
-        const float alpha = edge_adjoint(a, w, s, so[0], so[1], so[2], Go, xl_n, ds, nullptr);
+        float d = 1.0f;
+        if constexpr (DROP) d = attn_factor(a.drop, dk, id & 0x7fffffffu);
+        const float alpha = edge_adjoint<DROP>(a, w, s, so[0], so[1], so[2], Go, xl_n, ds, nullptr, d);
 #pragma unroll
         for (int c = 0; c < GC; ++c) dxl[c] += fmaf(alpha, Go[c], ds[c]);
       }
@@ -344,7 +408,9 @@ __global__ void __launch_bounds__(GAT_BWD_THREADS) k_gat_bwd(GatArgs a) {
       }
       float s[GC], ds[GC];
       edge_pre(w, xr_n, xl_n, abar, s);
-      const float alpha = edge_adjoint(a, w, s, m_n, den_n, t_n, Gn, xl_n, ds, datt);
+      float d = 1.0f;
+      if constexpr (DROP) d = attn_factor(a.drop, dk, (uint64_t)a.drop.num_edges + (uint64_t)n);
+      const float alpha = edge_adjoint<DROP>(a, w, s, m_n, den_n, t_n, Gn, xl_n, ds, datt, d);
 #pragma unroll
       for (int c = 0; c < GC; ++c) {
         dxr[c] += ds[c];
@@ -1140,9 +1206,10 @@ __global__ void k_gat_prep(GatPrepArgs p) {
   }
 }
 
-#define GAT_SLOT_CASE(S, KERN, GRID, THREADS) \
-  case S:                                     \
-    KERN<S><<<GRID, THREADS, 0, stream>>>(a); \
+#define GAT_SLOT_CASE(S, KERN, GRID, THREADS)                  \
+  case S:                                                      \
+    if (a.drop.mode) KERN<S, true><<<GRID, THREADS, 0, stream>>>(a); \
+    else KERN<S, false><<<GRID, THREADS, 0, stream>>>(a);            \
     break;
 #define GAT_SLOT_LAUNCH(slot, KERN, GRID, THREADS) \
   switch (slot) {                                  \
@@ -1159,6 +1226,28 @@ __global__ void k_gat_prep(GatPrepArgs p) {
       dss2_set_error("GAT weight slot %d outside -1..%d", slot, GAT_SLOTS - 1); \
       return -1;                            \
   }
+
+// dss2_attn_drop_t -> kernel arguments; mode stays 0 (the DROP = false kernels) for a NULL descriptor, p = 0 or mode 0
+int fill_drop(const char* who, AttnDropArgs& d, const dss2_attn_drop_t* drop, int64_t num_edges) {
+  d = AttnDropArgs{};
+  if (!drop) return 0;
+  DSS2_CHECK_ARG(drop->p >= 0.0f && drop->p < 1.0f, "%s: attention dropout p %f outside [0, 1)", who, drop->p);
+  DSS2_CHECK_ARG(drop->mode >= 0 && drop->mode <= 2, "%s: attention dropout mode %d outside 0..2", who, drop->mode);
+  DSS2_CHECK_ARG(drop->mode != 1 || drop->rng_state, "%s: philox attention dropout needs rng_state", who);
+  DSS2_CHECK_ARG(drop->mode != 2 || drop->mask, "%s: mask attention dropout needs a mask", who);
+  DSS2_CHECK_ARG(drop->head < 0x10000u, "%s: head %u outside 0..65535", who, drop->head);
+  if (drop->p == 0.0f || drop->mode == 0) return 0;
+  d.mode = drop->mode;
+  d.scale = 1.0f / (float)(1.0 - (double)drop->p);
+  const double thr = (1.0 - (double)drop->p) * 4294967296.0;
+  d.keep_thr = thr >= 4294967295.0 ? 0xffffffffu : (uint32_t)thr;
+  d.layer_uid = drop->layer_uid;
+  d.head = drop->head;
+  d.rng = drop->rng_state;
+  d.mask = drop->mask;
+  d.num_edges = num_edges;
+  return 0;
+}
 
 int grid_for(int64_t n, int threads) { return (int)max((int64_t)1, min((int64_t)dss2_sm_count() * 8, (n + threads - 1) / threads)); }
 
@@ -1196,12 +1285,13 @@ extern "C" size_t dss2_gat_ws_bytes(int64_t num_nodes) { return (size_t)num_node
 static int gat_fwd_impl(int slot, const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe,
                         const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b,
                         const float* lin_edge_w, const float* att, const float* bias, float att_slope, int act, float act_slope,
-                        float* y, void* stream_) {
+                        const dss2_attn_drop_t* drop, float* y, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   GatArgs a = {};
   if (fill_args("dss2_gat_fwd", a, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias,
                 att_slope, act, act_slope, slot))
     return -1;
+  if (fill_drop("dss2_gat_fwd", a.drop, drop, g->num_edges)) return -1;
   DSS2_CHECK_ARG(y && ((uintptr_t)y & 15) == 0, "dss2_gat_fwd: y must be a 16-byte aligned [Nt, 8] buffer");
   if (g->num_nodes == 0) return 0;
   a.y = y;
@@ -1215,7 +1305,31 @@ extern "C" int dss2_gat_fwd(const dss2_graph_t* g, const float* x, int64_t x_str
                             const float* lin_edge_w, const float* att, const float* bias, float att_slope, int act, float act_slope,
                             float* y, void* stream_) {
   return gat_fwd_impl(-1, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias, att_slope, act,
-                      act_slope, y, stream_);
+                      act_slope, nullptr, y, stream_);
+}
+
+extern "C" int dss2_gat_fwd_drop(const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe,
+                                 int slot, const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b,
+                                 const float* lin_edge_w, const float* att, const float* bias, float att_slope, int act, float act_slope,
+                                 const dss2_attn_drop_t* drop, float* y, void* stream_) {
+  return gat_fwd_impl(slot, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias, att_slope, act,
+                      act_slope, drop, y, stream_);
+}
+
+extern "C" int dss2_attn_drop_mask(const dss2_attn_drop_t* drop, int64_t num_edges, int64_t num_nodes, uint8_t* out, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  DSS2_CHECK_ARG(drop && out && num_edges >= 0 && num_nodes >= 0, "dss2_attn_drop_mask: null or negative argument");
+  AttnDropArgs d;
+  if (fill_drop("dss2_attn_drop_mask", d, drop, num_edges)) return -1;
+  const int64_t n = num_edges + num_nodes;
+  if (n == 0) return 0;
+  if (!d.mode) {   // no dropout: every coefficient kept
+    DSS2_CUDA(cudaMemsetAsync(out, 1, (size_t)n, stream));
+    return 0;
+  }
+  k_attn_drop_mask<<<grid_for(n, 256), 256, 0, stream>>>(d, n, out);
+  DSS2_LAUNCH_CHECK();
+  return 0;
 }
 
 // Weights of `count` layers -> constant-memory slots first .. first + count - 1: one layout kernel + one device-to-device copy (both
@@ -1248,7 +1362,7 @@ extern "C" int dss2_gat_fwd_slot(const dss2_graph_t* g, const float* x, int64_t 
                                  int slot, float att_slope, int act, float act_slope, float* y, void* stream_) {
   DSS2_CHECK_ARG(slot >= 0 && slot < GAT_SLOTS, "dss2_gat_fwd_slot: slot %d outside 0..%d", slot, GAT_SLOTS - 1);
   return gat_fwd_impl(slot, g, x, x_stride, edge_attr, ea_stride, fe, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, att_slope,
-                      act, act_slope, y, stream_);
+                      act, act_slope, nullptr, y, stream_);
 }
 
 // part_off[7]: offsets (floats, relative to `partials`) of the blocks [lin_l.w 64, lin_l.b 8, lin_r.w 64, lin_r.b 8, lin_edge.w 8 fe, att 8,
@@ -1256,13 +1370,14 @@ extern "C" int dss2_gat_fwd_slot(const dss2_graph_t* g, const float* x, int64_t 
 static int gat_bwd_impl(int slot, const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe,
                         const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b,
                         const float* lin_edge_w, const float* att, const float* bias, float att_slope, int act, float act_slope,
-                        const float* y, const float* grad_y, float* grad_x, float* node_ws, size_t node_ws_bytes, float* partials,
-                        int64_t partial_stride, const int64_t* part_off, void* stream_) {
+                        const dss2_attn_drop_t* drop, const float* y, const float* grad_y, float* grad_x, float* node_ws,
+                        size_t node_ws_bytes, float* partials, int64_t partial_stride, const int64_t* part_off, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   GatArgs a = {};
   if (fill_args("dss2_gat_bwd", a, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias,
                 att_slope, act, act_slope, slot))
     return -1;
+  if (fill_drop("dss2_gat_bwd", a.drop, drop, g->num_edges)) return -1;
   DSS2_CHECK_ARG(grad_y && node_ws && partials && part_off && (!(act & 0xff) || y), "dss2_gat_bwd: null argument");
   DSS2_CHECK_ARG(g->undirected == 1, "dss2_gat_bwd: needs a graph built from the one-way edge list with undirect=1 (out-edges of a bus are "
                  "found through the reversed entries)");
@@ -1307,7 +1422,18 @@ extern "C" int dss2_gat_bwd_ex(const dss2_graph_t* g, const float* x, int64_t x_
                                const float* y, const float* grad_y, float* grad_x, float* node_ws, size_t node_ws_bytes, float* partials,
                                int64_t partial_stride, const int64_t* part_off, void* stream_) {
   return gat_bwd_impl(-1, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias, att_slope, act,
-                      act_slope, y, grad_y, grad_x, node_ws, node_ws_bytes, partials, partial_stride, part_off, stream_);
+                      act_slope, nullptr, y, grad_y, grad_x, node_ws, node_ws_bytes, partials, partial_stride, part_off, stream_);
+}
+
+extern "C" int dss2_gat_bwd_drop(const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe,
+                                 int slot, const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b,
+                                 const float* lin_edge_w, const float* att, const float* bias, float att_slope, int act, float act_slope,
+                                 const dss2_attn_drop_t* drop, const float* y, const float* grad_y, float* grad_x, float* node_ws,
+                                 size_t node_ws_bytes, float* partials, int64_t partial_stride, const int64_t* part_off, void* stream_) {
+  const int64_t w = GC * GC, e0 = 2 * (w + GC);
+  const int64_t off[7] = {0, w, w + GC, 2 * w + GC, e0, e0 + (int64_t)GC * fe, e0 + (int64_t)GC * fe + GC};
+  return gat_bwd_impl(slot, g, x, x_stride, edge_attr, ea_stride, fe, lin_l_w, lin_l_b, lin_r_w, lin_r_b, lin_edge_w, att, bias, att_slope, act,
+                      act_slope, drop, y, grad_y, grad_x, node_ws, node_ws_bytes, partials, partial_stride, part_off ? part_off : off, stream_);
 }
 
 // the backward of a layer whose weights sit in constant-memory slot `slot` (part_off as in dss2_gat_bwd_ex; NULL: the standard partial row)
@@ -1319,7 +1445,8 @@ extern "C" int dss2_gat_bwd_slot(const dss2_graph_t* g, const float* x, int64_t 
   const int64_t w = GC * GC, e0 = 2 * (w + GC);
   const int64_t off[7] = {0, w, w + GC, 2 * w + GC, e0, e0 + (int64_t)GC * fe, e0 + (int64_t)GC * fe + GC};
   return gat_bwd_impl(slot, g, x, x_stride, edge_attr, ea_stride, fe, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, att_slope,
-                      act, act_slope, y, grad_y, grad_x, node_ws, node_ws_bytes, partials, partial_stride, part_off ? part_off : off, stream_);
+                      act, act_slope, nullptr, y, grad_y, grad_x, node_ws, node_ws_bytes, partials, partial_stride, part_off ? part_off : off,
+                      stream_);
 }
 
 // partial row: [lin_l.w 64 | lin_l.b 8 | lin_r.w 64 | lin_r.b 8 | lin_edge.w 8 fe | att 8 | bias 8]
@@ -1618,7 +1745,7 @@ extern "C" int dss2_lin8_bwd(int64_t num_nodes, int M, int weight_is_out_by_in, 
 // gnn_dsse(model='fagcn'): FAConv (networks.py:44-50; torch_geometric.nn.conv.FAConv) at width 8 on the one-way edge list:
 //   out[i] = sum_{j -> i} tanh(att_l . x[j] + att_r . x[i]) * dinv[j] dinv[i] * x[j]  (+ the self loop, appended last)  + eps * x_0[i]
 // followed by the model's non-linearity (fused here).  Thread per bus; the attention logits of the neighbours are recomputed from their
-// rows (8 FMAs) instead of stored.  FAConv's own dropout acts on the attention coefficients; the kernels cover dropout = 0 (the default).
+// rows (8 FMAs) instead of stored.  FAConv's own dropout acts on the attention coefficient tanh(.) (DROP kernels, edge keys as for GATv2).
 // -------------------------------------------------------------------------------------------------
 namespace {
 struct FaArgs {
@@ -1640,6 +1767,7 @@ struct FaArgs {
   float* acc;            // bwd, optional: acc[n] += eps * gz[n]  (the x_0 path)
   float* partials;       // bwd: per-CTA partial sums: [0, 8) att_l, [8, 16) att_r
   int64_t partial_stride;
+  AttnDropArgs drop;     // read by the DROP = true kernels only
 };
 __device__ __forceinline__ void fa_row(const float* p, float (&v)[GC]) {
 #pragma unroll
@@ -1658,11 +1786,14 @@ __device__ __forceinline__ float fa_act_grad(int act, float slope, float y) {
   return 1.0f;
 }
 
+template <bool DROP>
 __global__ void __launch_bounds__(GAT_THREADS) k_fa_fwd(FaArgs a) {
   const dss2_graph_t& g = a.g;
   float wl[GC], wr[GC];
   fa_row(a.att_l, wl);
   fa_row(a.att_r, wr);
+  AttnKey dk = {};
+  if constexpr (DROP) dk = attn_key(a.drop);
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < g.num_nodes; i += (int64_t)gridDim.x * blockDim.x) {
     const float di = a.dinv[i];
     float xi[GC], acc[GC];
@@ -1675,12 +1806,16 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_fwd(FaArgs a) {
       const int64_t j = g.col[z];
       float xj[GC];
       fa_row(a.x + j * a.xs, xj);
-      const float coef = tanhf(fa_dot(xj, wl) + ar) * (a.dinv[j] * di);
+      float t = tanhf(fa_dot(xj, wl) + ar);
+      if constexpr (DROP) t *= attn_factor(a.drop, dk, g.eid[z]);
+      const float coef = t * (a.dinv[j] * di);
 #pragma unroll
       for (int c = 0; c < GC; ++c) acc[c] = fmaf(coef, xj[c], acc[c]);
     }
     if (a.self_loops) {
-      const float coef = tanhf(fa_dot(xi, wl) + ar) * (di * di);
+      float t = tanhf(fa_dot(xi, wl) + ar);
+      if constexpr (DROP) t *= attn_factor(a.drop, dk, (uint64_t)a.drop.num_edges + (uint64_t)i);
+      const float coef = t * (di * di);
 #pragma unroll
       for (int c = 0; c < GC; ++c) acc[c] = fmaf(coef, xi[c], acc[c]);
     }
@@ -1702,12 +1837,16 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_fwd(FaArgs a) {
 // adjoint: with gz = grad_y * act'(y) and, per edge j -> i, t = tanh(al[j] + ar[i]), c = dinv[j] dinv[i], q = (1 - t^2) c (gz[i] . x[j]):
 //   grad_x[j] += t c gz[i] + q att_l,   grad_x[i] += q att_r,   grad_att_l += q x[j],   grad_att_r += q x[i].
 // A thread owns bus n: its in-edges give the att_r terms, its out-edges (same CSR row, flagged) the att_l terms and the message adjoint.
+// DROP: c includes the edge's dropout factor d (tc = t d c, q = (1 - t^2) c d (gz[i] . x[j])); the formulas above hold unchanged.
+template <bool DROP>
 __global__ void __launch_bounds__(GAT_THREADS) k_fa_bwd(FaArgs a) {
   const dss2_graph_t& g = a.g;
   __shared__ float red[GAT_THREADS / 32][2 * GC];
   float wl[GC], wr[GC], dwl[GC], dwr[GC];
   fa_row(a.att_l, wl);
   fa_row(a.att_r, wr);
+  AttnKey dk = {};
+  if constexpr (DROP) dk = attn_key(a.drop);
 #pragma unroll
   for (int c = 0; c < GC; ++c) dwl[c] = dwr[c] = 0.0f;
   for (int64_t n = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; n < g.num_nodes; n += (int64_t)gridDim.x * blockDim.x) {
@@ -1729,7 +1868,8 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_bwd(FaArgs a) {
       const int64_t m = g.col[z];
       float xm[GC];
       fa_row(a.x + m * a.xs, xm);
-      const float c = a.dinv[m] * dn;
+      float c = a.dinv[m] * dn;
+      if constexpr (DROP) c *= attn_factor(a.drop, dk, g.eid[z] & 0x7fffffffu);
       if (g.eid[z] >> 31) {   // n -> m
         float gzm[GC];
 #pragma unroll
@@ -1745,7 +1885,9 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_bwd(FaArgs a) {
       }
     }
     if (a.self_loops) {
-      const float t = tanhf(al_n + ar_n), c = dn * dn;
+      const float t = tanhf(al_n + ar_n);
+      float c = dn * dn;
+      if constexpr (DROP) c *= attn_factor(a.drop, dk, (uint64_t)a.drop.num_edges + (uint64_t)n);
       const float tc = t * c, q = (1.0f - t * t) * c * fa_dot(gzn, xn);
 #pragma unroll
       for (int k = 0; k < GC; ++k) gx[k] = fmaf(tc, gzn[k], gx[k]);
@@ -1801,26 +1943,35 @@ int fa_fill(const char* who, FaArgs& a, const dss2_graph_t* g, const float* dinv
 }
 }  // namespace
 
-extern "C" int dss2_fa_fwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* x0,
-                           int64_t x0_stride, const float* att_l, const float* att_r, float eps, int act, float slope, float* y,
-                           void* stream_) {
+extern "C" int dss2_fa_fwd_drop(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* x0,
+                                int64_t x0_stride, const float* att_l, const float* att_r, float eps, int act, float slope,
+                                const dss2_attn_drop_t* drop, float* y, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   FaArgs a = {};
   if (fa_fill("dss2_fa_fwd", a, g, dinv, self_loops, x, x_stride, x0, x0_stride, att_l, att_r, eps, act, slope)) return -1;
+  if (fill_drop("dss2_fa_fwd", a.drop, drop, g->num_edges)) return -1;
   DSS2_CHECK_ARG(y && ((uintptr_t)y & 15) == 0, "dss2_fa_fwd: y missing or unaligned");
   if (g->num_nodes == 0) return 0;
   a.y = y;
-  k_fa_fwd<<<grid_for(g->num_nodes, GAT_THREADS), GAT_THREADS, 0, stream>>>(a);
+  if (a.drop.mode) k_fa_fwd<true><<<grid_for(g->num_nodes, GAT_THREADS), GAT_THREADS, 0, stream>>>(a);
+  else k_fa_fwd<false><<<grid_for(g->num_nodes, GAT_THREADS), GAT_THREADS, 0, stream>>>(a);
   DSS2_LAUNCH_CHECK();
   return 0;
 }
 
-extern "C" int dss2_fa_bwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* att_l,
-                           const float* att_r, float eps, int act, float slope, const float* y, const float* grad_y, float* grad_x,
-                           float* acc_x0, float* partials, int64_t partial_stride, void* stream_) {
+extern "C" int dss2_fa_fwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* x0,
+                           int64_t x0_stride, const float* att_l, const float* att_r, float eps, int act, float slope, float* y,
+                           void* stream_) {
+  return dss2_fa_fwd_drop(g, dinv, self_loops, x, x_stride, x0, x0_stride, att_l, att_r, eps, act, slope, nullptr, y, stream_);
+}
+
+extern "C" int dss2_fa_bwd_drop(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* att_l,
+                                const float* att_r, float eps, int act, float slope, const dss2_attn_drop_t* drop, const float* y,
+                                const float* grad_y, float* grad_x, float* acc_x0, float* partials, int64_t partial_stride, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   FaArgs a = {};
   if (fa_fill("dss2_fa_bwd", a, g, dinv, self_loops, x, x_stride, x, x_stride, att_l, att_r, eps, act, slope)) return -1;
+  if (fill_drop("dss2_fa_bwd", a.drop, drop, g->num_edges)) return -1;
   DSS2_CHECK_ARG(grad_y && grad_x && partials && (!act || y) && ((uintptr_t)grad_x & 15) == 0, "dss2_fa_bwd: null or unaligned argument");
   a.yout = y;
   a.gy = grad_y;
@@ -1828,7 +1979,16 @@ extern "C" int dss2_fa_bwd(const dss2_graph_t* g, const float* dinv, int self_lo
   a.acc = acc_x0;
   a.partials = partials;
   a.partial_stride = partial_stride;
-  k_fa_bwd<<<dss2_num_partials(), GAT_THREADS, 0, stream>>>(a);   // every partial row is written (idle CTAs write zeros)
+  // every partial row is written (idle CTAs write zeros)
+  if (a.drop.mode) k_fa_bwd<true><<<dss2_num_partials(), GAT_THREADS, 0, stream>>>(a);
+  else k_fa_bwd<false><<<dss2_num_partials(), GAT_THREADS, 0, stream>>>(a);
   DSS2_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int dss2_fa_bwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* att_l,
+                           const float* att_r, float eps, int act, float slope, const float* y, const float* grad_y, float* grad_x,
+                           float* acc_x0, float* partials, int64_t partial_stride, void* stream_) {
+  return dss2_fa_bwd_drop(g, dinv, self_loops, x, x_stride, att_l, att_r, eps, act, slope, nullptr, y, grad_y, grad_x, acc_x0, partials,
+                          partial_stride, stream_);
 }

@@ -28,8 +28,14 @@ class GraphStruct(Structure):
     ]
 
 
+class AttnDrop(Structure):
+    """Mirror of `dss2_attn_drop_t` (attention dropout of one GATv2Conv / FAConv layer and head)."""
+    _fields_ = [("p", c_float), ("mode", c_int), ("rng_state", c_void_p), ("layer_uid", c_uint32), ("head", c_uint32), ("mask", c_void_p)]
+
+
 _P = c_void_p
 _G = POINTER(GraphStruct)
+_D = POINTER(AttnDrop)
 _SIGNATURES = {
     "dss2_last_error": (c_char_p, []),
     "dss2_version": (c_int, []),
@@ -100,6 +106,12 @@ _SIGNATURES = {
     "dss2_lin8_bwd": (c_int, [c_int64, c_int, c_int, _P, _P, _P, c_int, c_float, _P, _P, _P, _P, _P, c_float, _P, c_int64, c_int64, _P]),
     "dss2_fa_fwd": (c_int, [_G, _P, c_int, _P, c_int64, _P, c_int64, _P, _P, c_float, c_int, c_float, _P, _P]),
     "dss2_fa_bwd": (c_int, [_G, _P, c_int, _P, c_int64, _P, _P, c_float, c_int, c_float, _P, _P, _P, _P, _P, c_int64, _P]),
+    "dss2_gat_fwd_drop": (c_int, [_G, _P, c_int64, _P, c_int64, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_float, c_int, c_float, _D, _P, _P]),
+    "dss2_gat_bwd_drop": (c_int, [_G, _P, c_int64, _P, c_int64, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, c_float, c_int, c_float, _D,
+                                  _P, _P, _P, _P, c_size_t, _P, c_int64, _P, _P]),
+    "dss2_fa_fwd_drop": (c_int, [_G, _P, c_int, _P, c_int64, _P, c_int64, _P, _P, c_float, c_int, c_float, _D, _P, _P]),
+    "dss2_fa_bwd_drop": (c_int, [_G, _P, c_int, _P, c_int64, _P, _P, c_float, c_int, c_float, _D, _P, _P, _P, _P, _P, c_int64, _P]),
+    "dss2_attn_drop_mask": (c_int, [_D, c_int64, c_int64, _P, _P]),
     "dss2_mlp2_fwd": (c_int, [c_int64, _P, c_int, _P, _P, c_int, _P, _P, c_int, _P, _P, _P]),
     "dss2_mlp2_bwd": (c_int, [c_int64, _P, c_int, _P, c_int, _P, c_int, _P, _P, _P, _P, _P, c_int64, _P]),
     "dss2_mlp2_nh_supported": (c_int, [c_int, c_int, c_int]),
@@ -144,6 +156,15 @@ def check(rc, what):
 def ptr(t):
     """Device pointer of a tensor (None -> NULL)."""
     return None if t is None else c_void_p(t.data_ptr())
+
+
+def attn_drop(p, layer_uid, head=0, rng_state=None, mask=None):
+    """`dss2_attn_drop_t *` of one layer and head: the caller's mask (uint8 [Et + Nt]) when given, else the Philox stream of the device
+    {seed, step} `rng_state`; None (no dropout) when p == 0 or neither is given."""
+    if p == 0.0 or (rng_state is None and mask is None):
+        return None
+    return ctypes.pointer(AttnDrop(float(p), 2 if mask is not None else 1, None if rng_state is None else rng_state.data_ptr(), layer_uid, head,
+                                   None if mask is None else mask.data_ptr()))
 
 
 def stream():

@@ -14,7 +14,7 @@ import torch
 
 from . import _lib
 from .head import head_bwd, head_fwd
-from .ops import ParamPack, _align4, require_cuda, resolve_graph, stage_rows
+from .ops import ParamPack, _align4, fresh_rng_state, require_cuda, resolve_graph, stage_rows
 
 GAT_C = 8   # channels the kernels are built for (dim_feat of dss2_run.py:73)
 GAT_SLOTS = 8   # constant-memory weight slots of csrc/gat.cu
@@ -32,6 +32,7 @@ class GATSpec:
     act: str = "leaky_relu"   # nonlin of networks.py:130-137: 'leaky_relu' | 'relu' | 'tanh'
     self_loops: bool = True   # add_self_loops of the GATv2 layers (networks.py:145)
     heads: int = 1            # > 1: concat=False (mean over the heads)
+    dropout: float = 0.0      # attention dropout of the GATv2 layers (networks.py:145-146), applied when the caller asks for it
 
     @property
     def act_code(self):
@@ -185,7 +186,13 @@ class GATRunner:
             b["partials"] = torch.zeros(self.num_partials, self.flat_size, **f32)
         return b
 
-    def forward(self, graph, x, xs, ea, eas, flat, bufs):
+    def _drop(self, l, h, rng_state, masks):
+        return _lib.attn_drop(self.spec.dropout, l, h, rng_state, None if masks is None else masks[l][h])
+
+    def forward(self, graph, x, xs, ea, eas, flat, bufs, rng_state=None, masks=None):
+        """Attention dropout (p = spec.dropout) is applied when the caller passes the device {seed, step} `rng_state` (Philox, layer uid =
+        layer index, one stream per head) or `masks` (per layer uint8 [heads, Et + Nt], dss2_attn_drop_t's edge-key layout); the backward
+        must get the same."""
         sp, lib, st = self.spec, self.lib, _lib.stream()
         g = graph.ref
         H = sp.heads
@@ -196,31 +203,31 @@ class GATRunner:
             self.upload(flat)
         for l in range(sp.n_conv):
             xin, stride = (x, xs) if l == 0 else (bufs["acts"][l - 1], GAT_C)
-            if slots:
-                _lib.check(lib.dss2_gat_fwd_slot(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, l, sp.att_slope, sp.act_code,
-                                                 sp.act_slope, _lib.ptr(bufs["acts"][l]), st), "dss2_gat_fwd_slot")
-                continue
             if H > 1:
                 raw = bufs["raw"][l]
                 for h in range(H):
-                    _lib.check(lib.dss2_gat_fwd(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, *self._head(flat, l, h), sp.att_slope,
-                                                sp.act_code & 0x100, 0.0, _lib.ptr(raw[h]), st), "dss2_gat_fwd")
+                    _lib.check(lib.dss2_gat_fwd_drop(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, -1, *self._head(flat, l, h),
+                                                     sp.att_slope, sp.act_code & 0x100, 0.0, self._drop(l, h, rng_state, masks), _lib.ptr(raw[h]), st),
+                               "dss2_gat_fwd_drop")
                 # y = act(sum_h raw_h (I / H) + bias)
                 _lib.check(lib.dss2_lin8_fwd(graph.num_nodes, H, 1, self._arr([raw[h] for h in range(H)]), self._strides(H),
                                              self._p(flat, "_mean_blocks"), self._p(flat, f"model.module_{2 * l}.bias"), self._lin8_act,
                                              sp.act_slope, _lib.ptr(bufs["acts"][l]), st), "dss2_lin8_fwd")
                 continue
-            _lib.check(lib.dss2_gat_fwd(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, *self._layer(flat, l), sp.att_slope, sp.act_code,
-                                        sp.act_slope, _lib.ptr(bufs["acts"][l]), st), "dss2_gat_fwd")
+            # slots: the weights are immediate operands from constant-memory slot l (the pointers are not read)
+            _lib.check(lib.dss2_gat_fwd_drop(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, l if slots else -1, *self._layer(flat, l),
+                                             sp.att_slope, sp.act_code, sp.act_slope, self._drop(l, 0, rng_state, masks), _lib.ptr(bufs["acts"][l]),
+                                             st), "dss2_gat_fwd_drop")
         i = 2 * sp.n_conv
         head_fwd(lib, graph.num_nodes, _lib.ptr(bufs["acts"][sp.n_conv - 1]), GAT_C, self._p(flat, f"model.module_{i}.weight"),
                  self._p(flat, f"model.module_{i}.bias"), sp.dim_dense, self._p(flat, f"model.module_{i + 1}.weight"),
                  self._p(flat, f"model.module_{i + 1}.bias"), sp.dim_out, _lib.ptr(bufs["h"]), _lib.ptr(bufs["out"]), st)
         return bufs["out"]
 
-    def backward(self, graph, x, xs, ea, eas, flat, bufs, grad_out, flat_grad, need_gx=False, uploaded=False):
+    def backward(self, graph, x, xs, ea, eas, flat, bufs, grad_out, flat_grad, need_gx=False, uploaded=False, rng_state=None, masks=None):
         """grad_out [Nt, dim_out] dense -> flat parameter gradient (and grad wrt x when need_gx).  uploaded: the constant-memory slots
-        still hold this model's weights (the captured step: forward and backward of one step, nothing in between)."""
+        still hold this model's weights (the captured step: forward and backward of one step, nothing in between).  rng_state / masks:
+        those of the forward."""
         sp, lib, st = self.spec, self.lib, _lib.stream()
         g = graph.ref
         slots = self.use_slots()
@@ -254,10 +261,11 @@ class GATRunner:
                            "dss2_lin8_bwd")
                 for h in range(H):
                     offs = (ctypes.c_int64 * 7)(*[o - base for o in self._head_offsets(l, h)])
-                    _lib.check(lib.dss2_gat_bwd_ex(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, *self._head(flat, l, h), sp.att_slope,
-                                                   sp.act_code & 0x100, 0.0, _lib.ptr(raw[h]), _lib.ptr(graw[h]), _lib.ptr(gxh[h]) if want_gx else None,
-                                                   _lib.ptr(bufs["ws"]), bufs["ws"].numel() * 4, pp(f"model.module_{2 * l}.lin_l.weight"), pstride,
-                                                   offs, st), "dss2_gat_bwd_ex")
+                    _lib.check(lib.dss2_gat_bwd_drop(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, -1, *self._head(flat, l, h),
+                                                     sp.att_slope, sp.act_code & 0x100, 0.0, self._drop(l, h, rng_state, masks), _lib.ptr(raw[h]),
+                                                     _lib.ptr(graw[h]), _lib.ptr(gxh[h]) if want_gx else None, _lib.ptr(bufs["ws"]),
+                                                     bufs["ws"].numel() * 4, pp(f"model.module_{2 * l}.lin_l.weight"), pstride, offs, st),
+                               "dss2_gat_bwd_drop")
                 if want_gx:     # grad_x = sum over the heads (identity blocks = H * (I / H): scale folded into one more 8x8 pass)
                     _lib.check(lib.dss2_lin8_fwd(graph.num_nodes, H, 1, self._arr([gxh[h] for h in range(H)]), self._strides(H),
                                                  self._p(flat, "_mean_blocks"), None, 0, 0.0, _lib.ptr(gx), st), "dss2_lin8_fwd")
@@ -265,17 +273,10 @@ class GATRunner:
                 gy = gx
                 gx_out = gx
                 continue
-            if slots:
-                _lib.check(lib.dss2_gat_bwd_slot(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, l, sp.att_slope, sp.act_code, sp.act_slope,
-                                                 _lib.ptr(bufs["acts"][l]), _lib.ptr(gy), _lib.ptr(gx), _lib.ptr(bufs["ws"]), bufs["ws"].numel() * 4,
-                                                 pp(f"model.module_{2 * l}.lin_l.weight"), pstride, self._layer_offsets(l), st), "dss2_gat_bwd_slot")
-                gy = gx
-                gx_out = gx
-                continue
-            _lib.check(lib.dss2_gat_bwd_ex(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, *self._layer(flat, l), sp.att_slope, sp.act_code,
-                                           sp.act_slope, _lib.ptr(bufs["acts"][l]), _lib.ptr(gy), _lib.ptr(gx), _lib.ptr(bufs["ws"]),
-                                           bufs["ws"].numel() * 4, pp(f"model.module_{2 * l}.lin_l.weight"), pstride, self._layer_offsets(l), st),
-                       "dss2_gat_bwd_ex")
+            _lib.check(lib.dss2_gat_bwd_drop(g, _lib.ptr(xin), stride, _lib.ptr(ea), eas, sp.edge_dim, l if slots else -1, *self._layer(flat, l),
+                                             sp.att_slope, sp.act_code, sp.act_slope, self._drop(l, 0, rng_state, masks), _lib.ptr(bufs["acts"][l]),
+                                             _lib.ptr(gy), _lib.ptr(gx), _lib.ptr(bufs["ws"]), bufs["ws"].numel() * 4,
+                                             pp(f"model.module_{2 * l}.lin_l.weight"), pstride, self._layer_offsets(l), st), "dss2_gat_bwd_drop")
             gy = gx
             gx_out = gx
         _lib.check(lib.dss2_reduce_partials(_lib.ptr(part), pstride, self.num_partials, self.flat_size, _lib.ptr(flat_grad), 0, st),
@@ -285,39 +286,48 @@ class GATRunner:
 
 class _GATFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, edge_attr, edge_index, runner, pack, names, *params):
+    def forward(ctx, x, edge_attr, edge_index, runner, pack, names, drop, masks, *params):
         require_cuda()
         out_device = x.device
         named = dict(zip(names, params))
         xg, xs = stage_rows(x)
         eag, eas = stage_rows(edge_attr)
         graph = resolve_graph(edge_index, xg.size(0))
+        rng_state = None
         with torch.cuda.device(xg.device):
+            if drop and masks is not None:
+                masks = [m.to(device=xg.device, dtype=torch.uint8).contiguous() for m in masks]
+            elif drop:
+                rng_state = fresh_rng_state(xg.device)
+            else:
+                masks = None
             flat = pack.gather(named)
             bufs = runner.alloc(xg.size(0), xg.device, need_grad=any(ctx.needs_input_grad))   # False under torch.no_grad()
-            out = runner.forward(graph, xg, xs, eag, eas, flat, bufs)
+            out = runner.forward(graph, xg, xs, eag, eas, flat, bufs, rng_state=rng_state, masks=masks)
         ctx.runner, ctx.pack, ctx.names, ctx.graph, ctx.params = runner, pack, names, graph, params
-        ctx.saved = (xg, xs, eag, eas, flat, bufs)
+        ctx.saved = (xg, xs, eag, eas, flat, bufs, rng_state, masks)
         ctx.x_needs_grad, ctx.x_shape, ctx.x_device = x.requires_grad, x.shape, x.device
         result = out.clone()
         return result if out_device.type == "cuda" else result.to(out_device)
 
     @staticmethod
     def backward(ctx, grad_out):
-        xg, xs, eag, eas, flat, bufs = ctx.saved
+        xg, xs, eag, eas, flat, bufs, rng_state, masks = ctx.saved
         runner = ctx.runner
         go = grad_out.to(device=xg.device, dtype=torch.float32).contiguous()
         with torch.cuda.device(xg.device):
             flat_grad = torch.empty(runner.flat_size, dtype=torch.float32, device=xg.device)
-            gx = runner.backward(ctx.graph, xg, xs, eag, eas, flat, bufs, go, flat_grad, need_gx=ctx.x_needs_grad)
+            gx = runner.backward(ctx.graph, xg, xs, eag, eas, flat, bufs, go, flat_grad, need_gx=ctx.x_needs_grad, rng_state=rng_state, masks=masks)
         grads = ctx.pack.scatter_grads(flat_grad, dict(zip(ctx.names, ctx.params)))
         gx_ret = gx.clone().to(ctx.x_device) if ctx.x_needs_grad else None
-        return (gx_ret, None, None, None, None, None, *grads)
+        return (gx_ret, None, None, None, None, None, None, None, *grads)
 
 
-def gat_apply(runner, pack, named_params, x, edge_index, edge_attr):
+def gat_apply(runner, pack, named_params, x, edge_index, edge_attr, drop=False, masks=None):
+    """drop: apply the attention dropout of runner.spec (training mode) - with `masks` (per layer uint8 [heads, Et + Nt], 1 = keep) when
+    given, else with a fresh Philox seed from torch's global generator (so torch.manual_seed makes runs repeatable)."""
     names = tuple(named_params.keys())
-    return _GATFunction.apply(x, edge_attr, edge_index, runner, pack, names, *named_params.values())
+    return _GATFunction.apply(x, edge_attr, edge_index, runner, pack, names, drop, masks, *named_params.values())
 
 
 def make_machinery(spec):

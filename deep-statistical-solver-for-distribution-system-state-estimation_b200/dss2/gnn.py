@@ -1,5 +1,5 @@
 """Host side of gnn_dsse (reference networks.py:11-69, the rest of SURVEY.md 8f-1): `model='gcn2'` (GCN2Conv stack, the default),
-`model='fagcn'` (FAConv stack, dropout 0) and `model='tagcn'` (TAGConv stack) at width dim_feat == 8, followed by Linear(dim_feat, dim_dense), Linear(dim_dense, dim_out).
+`model='fagcn'` (FAConv stack, with its attention dropout) and `model='tagcn'` (TAGConv stack) at width dim_feat == 8, followed by Linear(dim_feat, dim_dense), Linear(dim_dense, dim_out).
 Spec, flat parameter layout under the names named_parameters() reports (`model.module_{2l}.weight1`, `.att_l.weight`, `.att_r.weight`, `.lins.{k}.weight`,
 `model.module_{2l}.bias`, the head), launch sequence, autograd bridge.  All arithmetic is in csrc/gat.cu (k_gcn_dinv, k_prop8,
 k_lin8_fwd/bwd, k_fa_fwd/bwd, k_outer_reduce, the mlp2 head); there is no CPU fallback.
@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from .head import head_bwd, head_fwd
-from .ops import ParamPack, _align4, require_cuda, resolve_graph, stage_rows
+from .ops import ParamPack, _align4, fresh_rng_state, require_cuda, resolve_graph, stage_rows
 
 C = 8
 ACTS = {"none": 0, "leaky_relu": 1, "relu": 2, "tanh": 3}
@@ -35,6 +35,7 @@ class GNNSpec:
     normalize: bool = True
     act: str = "leaky_relu"
     act_slope: float = 0.01
+    dropout: float = 0.0  # FAConv's attention dropout (networks.py:46), applied when the caller asks for it; gcn2 / tagcn ignore it
 
     @property
     def n_conv(self):
@@ -145,7 +146,12 @@ class GNNRunner:
         xin, stride = (x, xs) if l == 0 else (bufs["acts"][l - 1], C)
         return [xin] + [bufs["lev"][l, k] for k in range(sp.K)], [stride] + [C] * sp.K
 
-    def forward(self, graph, x, xs, flat, bufs):
+    def _drop(self, l, rng_state, masks):
+        return _lib.attn_drop(self.spec.dropout, l, 0, rng_state, None if masks is None else masks[l][0])
+
+    def forward(self, graph, x, xs, flat, bufs, rng_state=None, masks=None):
+        """fagcn: attention dropout (p = spec.dropout) when the caller passes the device {seed, step} `rng_state` (Philox, layer uid =
+        layer index) or `masks` (per layer uint8 [1, Et + Nt], dss2_attn_drop_t's edge-key layout); the backward must get the same."""
         sp, lib, st, g = self.spec, self.lib, _lib.stream(), graph.ref
         loops = 1 if (sp.self_loops and sp.model != "tagcn") else 0      # TAGConv: gcn_norm(add_self_loops=False)
         _lib.check(lib.dss2_gcn_dinv(g, loops, _lib.ptr(bufs["dinv"]), st), "dss2_gcn_dinv")
@@ -153,9 +159,9 @@ class GNNRunner:
             xin, stride = (x, xs) if l == 0 else (bufs["acts"][l - 1], C)
             if sp.model == "fagcn":
                 p = f"model.module_{2 * l}."
-                _lib.check(lib.dss2_fa_fwd(g, _lib.ptr(bufs["dinv"]), loops, _lib.ptr(xin), stride, _lib.ptr(x), xs, self._p(flat, p + "att_l.weight"),
-                                           self._p(flat, p + "att_r.weight"), sp.alpha, ACTS[sp.act], sp.act_slope, _lib.ptr(bufs["acts"][l]), st),
-                           "dss2_fa_fwd")
+                _lib.check(lib.dss2_fa_fwd_drop(g, _lib.ptr(bufs["dinv"]), loops, _lib.ptr(xin), stride, _lib.ptr(x), xs,
+                                                self._p(flat, p + "att_l.weight"), self._p(flat, p + "att_r.weight"), sp.alpha, ACTS[sp.act],
+                                                sp.act_slope, self._drop(l, rng_state, masks), _lib.ptr(bufs["acts"][l]), st), "dss2_fa_fwd_drop")
                 continue
             if sp.model == "gcn2":
                 # h = (1 - alpha) A x + alpha x_0   (GCN2Conv.forward: x.mul_(1 - alpha); x_0 = alpha * x_0; out = x.add_(x_0))
@@ -177,8 +183,8 @@ class GNNRunner:
                  self._p(flat, f"model.module_{i + 1}.bias"), sp.dim_out, _lib.ptr(bufs["h"]), _lib.ptr(bufs["out"]), st)
         return bufs["out"]
 
-    def backward(self, graph, x, xs, flat, bufs, grad_out, flat_grad):
-        """grad_out [Nt, dim_out] dense -> flat parameter gradient; returns grad wrt x [Nt, 8]."""
+    def backward(self, graph, x, xs, flat, bufs, grad_out, flat_grad, rng_state=None, masks=None):
+        """grad_out [Nt, dim_out] dense -> flat parameter gradient; returns grad wrt x [Nt, 8].  rng_state / masks: those of the forward."""
         sp, lib, st, g = self.spec, self.lib, _lib.stream(), graph.ref
         part, pstride = bufs["partials"], self.flat_size
         loops = 1 if (sp.self_loops and sp.model != "tagcn") else 0
@@ -197,10 +203,10 @@ class GNNRunner:
                 p = f"model.module_{2 * l}."
                 xin, stride = (x, xs) if l == 0 else (bufs["acts"][l - 1], C)
                 gx = bufs["g8"][(sp.n_conv - l) & 1]
-                _lib.check(lib.dss2_fa_bwd(g, _lib.ptr(bufs["dinv"]), loops, _lib.ptr(xin), stride, self._p(flat, p + "att_l.weight"),
-                                           self._p(flat, p + "att_r.weight"), sp.alpha, ACTS[sp.act], sp.act_slope, _lib.ptr(bufs["acts"][l]),
-                                           _lib.ptr(gy), _lib.ptr(gx), _lib.ptr(bufs["gx0"]) if sp.alpha != 0.0 else None,
-                                           pp(self.table[p + "att_l.weight"][0]), pstride, st), "dss2_fa_bwd")
+                _lib.check(lib.dss2_fa_bwd_drop(g, _lib.ptr(bufs["dinv"]), loops, _lib.ptr(xin), stride, self._p(flat, p + "att_l.weight"),
+                                                self._p(flat, p + "att_r.weight"), sp.alpha, ACTS[sp.act], sp.act_slope, self._drop(l, rng_state, masks),
+                                                _lib.ptr(bufs["acts"][l]), _lib.ptr(gy), _lib.ptr(gx), _lib.ptr(bufs["gx0"]) if sp.alpha != 0.0 else None,
+                                                pp(self.table[p + "att_l.weight"][0]), pstride, st), "dss2_fa_bwd_drop")
                 if l == 0 and sp.alpha != 0.0:
                     gx.add_(bufs["gx0"])          # the x_0 path (eps * sum_l grad_z_l) joins the gradient of the model input
                 gy = gx
@@ -236,7 +242,7 @@ class GNNRunner:
 
 class _GNNFunction(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, edge_index, runner, pack, names, *params):
+    def forward(ctx, x, edge_index, runner, pack, names, drop, masks, *params):
         require_cuda()
         out_device = x.device
         named = dict(zip(names, params))
@@ -246,32 +252,41 @@ class _GNNFunction(torch.autograd.Function):
         graph = resolve_graph(edge_index, xg.size(0))
         if graph.c.undirected != 1:
             raise _lib.Dss2Error("gnn_dsse expects the one-way edge list of the reference's data (from_bus -> to_bus)")
+        rng_state = None
         with torch.cuda.device(xg.device):
+            if drop and masks is not None:
+                masks = [m.to(device=xg.device, dtype=torch.uint8).contiguous() for m in masks]
+            elif drop:
+                rng_state = fresh_rng_state(xg.device)
+            else:
+                masks = None
             flat = pack.gather(named)
             bufs = runner.alloc(xg.size(0), xg.device, need_grad=any(ctx.needs_input_grad))
-            out = runner.forward(graph, xg, xs, flat, bufs)
+            out = runner.forward(graph, xg, xs, flat, bufs, rng_state=rng_state, masks=masks)
         ctx.runner, ctx.pack, ctx.names, ctx.graph, ctx.params = runner, pack, names, graph, params
-        ctx.saved = (xg, xs, flat, bufs)
+        ctx.saved = (xg, xs, flat, bufs, rng_state, masks)
         ctx.x_needs_grad, ctx.x_device = x.requires_grad, x.device
         result = out.clone()
         return result if out_device.type == "cuda" else result.to(out_device)
 
     @staticmethod
     def backward(ctx, grad_out):
-        xg, xs, flat, bufs = ctx.saved
+        xg, xs, flat, bufs, rng_state, masks = ctx.saved
         runner = ctx.runner
         go = grad_out.to(device=xg.device, dtype=torch.float32).contiguous()
         with torch.cuda.device(xg.device):
             flat_grad = torch.empty(runner.flat_size, dtype=torch.float32, device=xg.device)
-            gx = runner.backward(ctx.graph, xg, xs, flat, bufs, go, flat_grad)
+            gx = runner.backward(ctx.graph, xg, xs, flat, bufs, go, flat_grad, rng_state=rng_state, masks=masks)
         grads = ctx.pack.scatter_grads(flat_grad, dict(zip(ctx.names, ctx.params)))
         gx_ret = gx.clone().to(ctx.x_device) if ctx.x_needs_grad else None
-        return (gx_ret, None, None, None, None, *grads)
+        return (gx_ret, None, None, None, None, None, None, *grads)
 
 
-def gnn_apply(runner, pack, named_params, x, edge_index):
+def gnn_apply(runner, pack, named_params, x, edge_index, drop=False, masks=None):
+    """drop: apply FAConv's attention dropout of runner.spec (training mode) - with `masks` (per layer uint8 [1, Et + Nt], 1 = keep) when
+    given, else with a fresh Philox seed from torch's global generator."""
     names = tuple(named_params.keys())
-    return _GNNFunction.apply(x, edge_index, runner, pack, names, *named_params.values())
+    return _GNNFunction.apply(x, edge_index, runner, pack, names, drop, masks, *named_params.values())
 
 
 def make_machinery(spec):

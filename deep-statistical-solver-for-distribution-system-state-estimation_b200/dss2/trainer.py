@@ -182,7 +182,9 @@ class GraphedTrainer:
             out = self.runner.forward(self.graph, b["x"], 11, b["edge_attr"], 13, self.flat, self.bufs,
                                       drop_mode=1 if self.spec.p_drop > 0 else 0, rng_state=self.step_state, ea_uploaded=bool(pre))
         else:
-            out = self.runner.forward(self.graph, b["x"], 11, b["edge_attr"], 13, self.flat, self.bufs)
+            # GAT: the attention dropout of GATSpec.dropout (training mode) draws from the same device {seed, step} as the TAG dropout
+            kw = {"rng_state": self.step_state} if self.network == "gat" else {}
+            out = self.runner.forward(self.graph, b["x"], 11, b["edge_attr"], 13, self.flat, self.bufs, **kw)
         wls_args = (self.graph.ref, _lib.ptr(b["x"]), 11, _lib.ptr(b["edge_attr"]), 13, _lib.ptr(out), _lib.ptr(self.stats), *self.coefs,
                     _lib.ptr(b["vminmax"]), 1, _lib.ptr(self.loss), None, _lib.ptr(self.grad_out), _lib.ptr(self.wls_ws),
                     self.wls_ws.numel() * self.wls_ws.element_size(), st)
@@ -202,7 +204,8 @@ class GraphedTrainer:
                                  rng_state=self.step_state, bucket_hook=hook)
             reduced = self.runner.bucketed
         else:
-            kw = {"uploaded": True} if self.network == "gat" else {}      # GAT: the forward's constant-memory weight slots are still valid
+            # GAT: the forward's constant-memory weight slots are still valid, and the backward re-draws the forward's dropout masks
+            kw = {"uploaded": True, "rng_state": self.step_state} if self.network == "gat" else {}
             self.runner.backward(self.graph, b["x"], 11, b["edge_attr"], 13, self.flat, self.bufs, self.grad_out, self.flat_grad, **kw)
             reduced = False
         if self.world > 1 and not reduced:

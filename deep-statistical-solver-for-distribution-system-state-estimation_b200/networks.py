@@ -161,6 +161,18 @@ class SkipPFN(PFN):
     _sub = SkipMPN
 
 
+def _check_attn_dropout(p, who):
+    """Attention dropout probability as F.dropout accepts it (ValueError outside [0, 1]); p == 1 (every coefficient dropped) is not built.
+    p > 0 exists only as CUDA kernels (the masks are drawn inside them): without a CUDA device it is refused when the model is built."""
+    if p < 0. or p > 1.:
+        raise ValueError(f"dropout probability has to be between 0 and 1, but got {p}")
+    if p == 1.:
+        raise NotImplementedError(f"{who}: attention dropout p == 1 (every attention coefficient dropped) is not supported")
+    if p > 0. and not torch.cuda.is_available():
+        raise NotImplementedError(f"{who}: attention dropout runs in the CUDA kernels only and no CUDA device is available "
+                                  "(there is no CPU implementation)")
+
+
 class _GCN2Params(nn.Module):
     """Parameter holder with PyG GCN2Conv's name / shape / initialisation: `weight1` [channels, channels], glorot (shared_weights=True:
     no `weight2`).  The arithmetic is in the fused kernels (csrc/gat.cu)."""
@@ -185,8 +197,10 @@ class gnn_dsse(_LazyMachinery, nn.Module):
     (children `module_{i}`), `forward(x, edge_index)` with x_0 = x.  conv = GCN2Conv(channels, alpha=main_param, theta, shared_weights,
     cached, normalize, add_self_loops) for model='gcn2' (the default), FAConv(channels, eps=main_param, dropout, cached, normalize,
     add_self_loops) for model='fagcn', or TAGConv(channels, channels, K, bias, normalize) for model='tagcn'.  Built for what the
-    reference's defaults select (theta=None, shared_weights=True, normalize=True, dropout 0); the other settings raise.
+    reference's defaults select (theta=None, shared_weights=True, normalize=True); the other settings raise.  `dropout` is FAConv's
+    attention dropout (0 <= p < 1), active in train() only like PyG's; gcn2 and tagcn ignore it, as the reference does.
     `cached=True` is accepted and ignored: the normalisation is recomputed per batch."""
+    _dss2_attn_masks = None   # test hook (fagcn): per layer uint8 [1, Et + Nt] keep masks in the kernels' edge-key layout, consumed by the next forward
 
     def __init__(self, dim_feat, dim_dense, dim_out, num_layers, nonlin='leaky_relu', main_param=0.1, K=3, bias=True, dropout=0., theta=None,
                  shared_weights=True, cached=True, add_self_loops=True, normalize=True, model='gcn2'):
@@ -195,9 +209,8 @@ class gnn_dsse(_LazyMachinery, nn.Module):
             raise Exception('invalid activation type')
         if model not in ('gcn2', 'fagcn', 'tagcn'):
             raise Exception('invalid model type')
-        if model == 'fagcn' and dropout != 0.:
-            raise NotImplementedError("gnn_dsse(model='fagcn') kernels cover dropout=0 (FAConv's dropout acts on the attention coefficients, "
-                                      "networks.py:46; the reference default is 0)")
+        if model == 'fagcn':
+            _check_attn_dropout(dropout, "gnn_dsse(model='fagcn')")
         if theta is not None or not shared_weights or not normalize:
             raise NotImplementedError("gnn_dsse kernels cover theta=None, shared_weights=True, normalize=True (the reference's defaults)")
         self.channels, self.main_param, self.dim_out, self.K, self.dropout, self.bias = dim_feat, main_param, dim_out, K, dropout, bias
@@ -221,7 +234,8 @@ class gnn_dsse(_LazyMachinery, nn.Module):
             spec = gnn.GNNSpec(model=self.kind, dim_feat=self.channels, dim_dense=self.dim_dense, dim_out=self.dim_out,
                                num_layers=self.num_layers, alpha=float(self.main_param), K=self.K, bias=bool(self.bias),
                                self_loops=bool(self.add_self_loops), normalize=bool(self.normalize), act=self.nonlin_name,
-                               act_slope=float(getattr(self.nonlin, "negative_slope", 0.0)))
+                               act_slope=float(getattr(self.nonlin, "negative_slope", 0.0)),
+                               dropout=float(self.dropout) if self.kind == 'fagcn' else 0.0)
             m = gnn.make_machinery(spec)
             self.__dict__["_dss2_machinery"] = m
         return m
@@ -229,7 +243,9 @@ class gnn_dsse(_LazyMachinery, nn.Module):
     def forward(self, x, edge_index):
         from dss2 import gnn
         runner, pack = self._machinery()
-        return gnn.gnn_apply(runner, pack, self._named_params(), x, edge_index)
+        masks, self._dss2_attn_masks = self._dss2_attn_masks, None
+        drop = self.training and runner.spec.dropout > 0.      # FAConv: F.dropout(..., training=self.training)
+        return gnn.gnn_apply(runner, pack, self._named_params(), x, edge_index, drop=drop, masks=masks)
 
 
 class _GINEParams(nn.Module):
@@ -314,9 +330,11 @@ class GAT_DSSE(_LazyMachinery, nn.Module):
     """networks.py:113-156, the as-shipped default model of dss2_run.py:86: (num_layers - 1) x [GATv2Conv(dim_feat, dim_feat, heads,
     edge_dim, add_self_loops, fill 'mean') + LeakyReLU()], Linear(dim_feat, dim_dense), Linear(dim_dense, dim_out), wrapped in a PyG
     `Sequential` whose children are called `module_{i}` - kept, so that reference checkpoints (`model.module_0.att`, ...) load.
-    heads=1 (with either `concat`: one head concatenated = one head averaged) or heads 2..4 with concat=False (averaged heads),
-    attention dropout 0; `self_loops`, `slope` and the three `nonlin` choices are free.  heads > 1 with concat=True raises (the
-    reference's own stack cannot run it: channel mismatch)."""
+    heads=1 (with either `concat`: one head concatenated = one head averaged) or heads 2..4 with concat=False (averaged heads);
+    `self_loops`, `slope` and the three `nonlin` choices are free.  `dropout` (0 <= p < 1) is GATv2Conv's attention dropout, active in
+    train() only like PyG's (unlike the MPN family's always-on nn.Dropout); each forward draws a fresh Philox seed from torch's global
+    generator.  heads > 1 with concat=True raises (the reference's own stack cannot run it: channel mismatch)."""
+    _dss2_attn_masks = None   # test hook: per layer uint8 [heads, Et + Nt] keep masks in the kernels' edge-key layout, consumed by the next forward
 
     def __init__(self, dim_feat, dim_dense, dim_out, num_layers, edge_dim, heads=1, concat=True, slope=0.2, self_loops=True, dropout=0.,
                  nonlin='leaky_relu', model='gat'):
@@ -330,8 +348,7 @@ class GAT_DSSE(_LazyMachinery, nn.Module):
                                       "dim_feat -> heads * dim_feat channels while the next layer expects dim_feat (networks.py:144-147)")
         if not 1 <= heads <= 4:
             raise NotImplementedError("GAT_DSSE kernels support heads in 1..4 (dss2_run.py:79 uses 1)")
-        if dropout != 0.:
-            raise NotImplementedError("GAT_DSSE kernels are built for attention dropout 0 (dss2_run.py:86)")
+        _check_attn_dropout(dropout, "GAT_DSSE")
         self.dim_out, self.num_layers, self.dim_feat, self.dim_dense, self.edge_dim = dim_out, num_layers, dim_feat, dim_dense, edge_dim
         self.dim_hidden = self.channels = dim_feat
         self.heads, self.concat, self.slope, self.dropout, self.loop = heads, concat, slope, dropout, self_loops
@@ -352,7 +369,7 @@ class GAT_DSSE(_LazyMachinery, nn.Module):
             from dss2 import gat
             spec = gat.GATSpec(dim_feat=self.dim_feat, dim_dense=self.dim_dense, dim_out=self.dim_out, num_layers=self.num_layers,
                                edge_dim=self.edge_dim, att_slope=float(self.slope), act_slope=float(getattr(self.nonlin, "negative_slope", 0.0)),
-                               act=self.nonlin_name, self_loops=bool(self.loop), heads=int(self.heads))
+                               act=self.nonlin_name, self_loops=bool(self.loop), heads=int(self.heads), dropout=float(self.dropout))
             m = gat.make_machinery(spec)
             self.__dict__["_dss2_machinery"] = m
         return m
@@ -360,4 +377,6 @@ class GAT_DSSE(_LazyMachinery, nn.Module):
     def forward(self, x, edge_index, edge_attr):
         from dss2 import gat
         runner, pack = self._machinery()
-        return gat.gat_apply(runner, pack, self._named_params(), x, edge_index, edge_attr)
+        masks, self._dss2_attn_masks = self._dss2_attn_masks, None
+        drop = self.training and runner.spec.dropout > 0.      # GATv2Conv: F.dropout(alpha, training=self.training)
+        return gat.gat_apply(runner, pack, self._named_params(), x, edge_index, edge_attr, drop=drop, masks=masks)

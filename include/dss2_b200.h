@@ -414,7 +414,7 @@ int dss2_lin8_bwd(int64_t num_nodes, int M, int weight_is_out_by_in, const float
                   int act, float slope, const float* y, const float* grad_y, float* grad_z, float* const* grad_in, float* acc,
                   float acc_scale, float* partials, int64_t partial_stride, int64_t bias_offset, void* stream);
 
-/* gnn_dsse(model='fagcn') (networks.py:44-50, torch_geometric FAConv with dropout = 0) at width 8 on the one-way edge list:
+/* gnn_dsse(model='fagcn') (networks.py:44-50, torch_geometric FAConv; dropout: dss2_fa_fwd_drop below) at width 8 on the one-way edge list:
  *   y[i] = act( sum_{j -> i} tanh(att_l . x[j] + att_r . x[i]) dinv[j] dinv[i] x[j]  (+ self loop, last)  + eps x0[i] ).
  * dss2_fa_bwd: grad_x (adjoint of x, message and attention paths), optionally acc_x0 += eps * grad_z (the x_0 path), and per-CTA
  * partial sums of the attention gradients at partials[0..8) (att_l) and partials[8..16) (att_r), dss2_num_partials() rows. */
@@ -423,6 +423,48 @@ int dss2_fa_fwd(const dss2_graph_t* g, const float* dinv, int self_loops, const 
 int dss2_fa_bwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* att_l,
                 const float* att_r, float eps, int act, float slope, const float* y, const float* grad_y, float* grad_x,
                 float* acc_x0, float* partials, int64_t partial_stride, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Attention dropout of GATv2Conv (networks.py:145-146, `dropout` of GAT_DSSE) and FAConv (networks.py:46, `dropout` of
+ * gnn_dsse(model='fagcn')) in training mode: alpha = F.dropout(softmax_i(score), p) for GATv2, coef = F.dropout(tanh(.), p) * w for
+ * FAConv, every coefficient of a softmax segment - the appended self loop too - kept with probability 1 - p and scaled by 1 / (1 - p).
+ * Descriptor (host struct, one per layer and head):
+ *   p in [0, 1); mode 0 none, 1 counter-based Philox keyed by (seed, step) read from DEVICE memory rng_state[2] (graph-replay safe, as
+ *   dss2_tag_fwd) with layer_uid and head, 2 caller mask `mask` (uint8 [Et + Nt], 1 = keep).  p == 0 or mode 0 = no dropout.
+ *   Edge key of a coefficient: the one-way edge id e for a real edge, Et + i for the loop appended at bus i (mode 2: entries of
+ *   dropped input self loops are ignored, the loop entries are unused without add_self_loops).
+ * The forward and both backward passes re-draw the same bit wherever they visit a coefficient; nothing is stored between them.
+ * dss2_gat_fwd_drop / dss2_gat_bwd_drop: dss2_gat_fwd / dss2_gat_bwd_ex with a weight slot (slot >= 0: dss2_gat_upload's weights, the
+ *   pointers are ignored; -1: weights from the pointers) and a descriptor (NULL = none).  bwd: part_off NULL = the standard partial row.
+ * dss2_fa_fwd_drop / dss2_fa_bwd_drop: dss2_fa_fwd / dss2_fa_bwd with a descriptor.
+ * dss2_attn_drop_mask: writes the mask [Et + Nt] (1 = keep) that the descriptor applies, from the same device function as the layer
+ *   kernels (mode 1: what the Philox stream draws for this seed, step, layer_uid and head).
+ * All of them are capturable: no host synchronisation, no allocation.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dss2_attn_drop {
+  float p;
+  int mode;
+  const uint64_t* rng_state;
+  uint32_t layer_uid;
+  uint32_t head;
+  const uint8_t* mask;
+} dss2_attn_drop_t;
+int dss2_gat_fwd_drop(const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe, int slot,
+                      const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b, const float* lin_edge_w,
+                      const float* att, const float* bias, float att_slope, int act, float act_slope, const dss2_attn_drop_t* drop,
+                      float* y, void* stream);
+int dss2_gat_bwd_drop(const dss2_graph_t* g, const float* x, int64_t x_stride, const float* edge_attr, int64_t ea_stride, int fe, int slot,
+                      const float* lin_l_w, const float* lin_l_b, const float* lin_r_w, const float* lin_r_b, const float* lin_edge_w,
+                      const float* att, const float* bias, float att_slope, int act, float act_slope, const dss2_attn_drop_t* drop,
+                      const float* y, const float* grad_y, float* grad_x, float* node_ws, size_t node_ws_bytes, float* partials,
+                      int64_t partial_stride, const int64_t* part_off, void* stream);
+int dss2_fa_fwd_drop(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* x0,
+                     int64_t x0_stride, const float* att_l, const float* att_r, float eps, int act, float slope,
+                     const dss2_attn_drop_t* drop, float* y, void* stream);
+int dss2_fa_bwd_drop(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* att_l,
+                     const float* att_r, float eps, int act, float slope, const dss2_attn_drop_t* drop, const float* y,
+                     const float* grad_y, float* grad_x, float* acc_x0, float* partials, int64_t partial_stride, void* stream);
+int dss2_attn_drop_mask(const dss2_attn_drop_t* drop, int64_t num_edges, int64_t num_nodes, uint8_t* out, void* stream);
 
 #ifdef __cplusplus
 }
