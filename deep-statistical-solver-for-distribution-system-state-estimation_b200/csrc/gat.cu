@@ -1024,10 +1024,13 @@ __global__ void __launch_bounds__(GAT_BWD_THREADS) k_gine_bwd_b(GineArgs a) {
 // un-direct it), built from four small thread-per-bus kernels.  The CSR rows of dss2_graph_t hold the in-edges of a bus (entries
 // without the reversed flag, in edge order = PyG's scatter order) and, flagged, its out-edges: the transposed propagation of the
 // backward walks the same row.
+// self_loops = 1 is gcn_norm(add_self_loops=True), i.e. PyG's add_remaining_self_loops: the self loops of the input are dropped (an
+// entry with col == i) and exactly one loop of weight 1 per bus is appended last.  self_loops = 0 takes the edge list as given: an
+// input loop is an ordinary edge (TAGConv's gcn_norm(add_self_loops=False)).
 // -------------------------------------------------------------------------------------------------
 struct GnnArgs {
   dss2_graph_t g;
-  const float* dinv;     // [Nt] deg^-1/2 of gcn_norm (in-degree, + 1 with self loops), inf -> 0
+  const float* dinv;     // [Nt] deg^-1/2 of gcn_norm (in-degree; with self loops: input loops not counted, + 1), inf -> 0
   int self_loops;
   int transposed;
   const float* x;        // [Nt, >= 8], row stride xs
@@ -1042,12 +1045,13 @@ struct GnnArgs {
 __global__ void __launch_bounds__(GAT_THREADS) k_gcn_dinv(dss2_graph_t g, int self_loops, float* dinv) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < g.num_nodes; i += (int64_t)gridDim.x * blockDim.x) {
     int deg = self_loops ? 1 : 0;
-    for (int z = g.rowptr[i]; z < g.rowptr[i + 1]; ++z) deg += (g.eid[z] >> 31) ? 0 : 1;
+    for (int z = g.rowptr[i]; z < g.rowptr[i + 1]; ++z) deg += ((g.eid[z] >> 31) || (self_loops && g.col[z] == i)) ? 0 : 1;
     dinv[i] = deg > 0 ? 1.0f / sqrtf((float)deg) : 0.0f;   // deg.pow(-0.5), inf -> 0 (gcn_norm)
   }
 }
 
 // out[i] = scale * sum_{j -> i} dinv[j] dinv[i] x[j] (+ self loop last, as add_remaining_self_loops appends it) + add_scale * add[i];
+// with self loops the input loops (j == i) are skipped, in both directions.
 // transposed: the sum runs over the out-edges i -> j instead (adjoint of the propagation).  Every product / sum is rounded on its own
 // like the eager ops of the reference (no fused multiply-add).
 __global__ void __launch_bounds__(GAT_THREADS) k_prop8(GnnArgs a) {
@@ -1061,6 +1065,7 @@ __global__ void __launch_bounds__(GAT_THREADS) k_prop8(GnnArgs a) {
       const bool rev = g.eid[z] >> 31;
       if (rev != (a.transposed != 0)) continue;
       const int64_t j = g.col[z];
+      if (a.self_loops && j == i) continue;   // an input loop: replaced by the appended one
       const float w = __fmul_rn(a.dinv[j], di);
       const float* xj = a.x + j * a.xs;
 #pragma unroll
@@ -1746,6 +1751,7 @@ extern "C" int dss2_lin8_bwd(int64_t num_nodes, int M, int weight_is_out_by_in, 
 //   out[i] = sum_{j -> i} tanh(att_l . x[j] + att_r . x[i]) * dinv[j] dinv[i] * x[j]  (+ the self loop, appended last)  + eps * x_0[i]
 // followed by the model's non-linearity (fused here).  Thread per bus; the attention logits of the neighbours are recomputed from their
 // rows (8 FMAs) instead of stored.  FAConv's own dropout acts on the attention coefficient tanh(.) (DROP kernels, edge keys as for GATv2).
+// With self loops the input loops are skipped (add_remaining_self_loops), so their dropout keys are never read, as for GATv2.
 // -------------------------------------------------------------------------------------------------
 namespace {
 struct FaArgs {
@@ -1804,6 +1810,7 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_fwd(FaArgs a) {
     for (int z = g.rowptr[i]; z < g.rowptr[i + 1]; ++z) {
       if (g.eid[z] >> 31) continue;           // out-edge of i
       const int64_t j = g.col[z];
+      if (a.self_loops && j == i) continue;   // an input loop: replaced by the appended one
       float xj[GC];
       fa_row(a.x + j * a.xs, xj);
       float t = tanhf(fa_dot(xj, wl) + ar);
@@ -1866,6 +1873,7 @@ __global__ void __launch_bounds__(GAT_THREADS) k_fa_bwd(FaArgs a) {
     float q_l = 0.0f, q_r = 0.0f;   // sums of q over the out-edges (n is the source) and the in-edges (n is the target)
     for (int z = g.rowptr[n]; z < g.rowptr[n + 1]; ++z) {
       const int64_t m = g.col[z];
+      if (a.self_loops && m == n) continue;   // an input loop (its in- and its out-entry): replaced by the appended one
       float xm[GC];
       fa_row(a.x + m * a.xs, xm);
       float c = a.dinv[m] * dn;

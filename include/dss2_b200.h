@@ -397,9 +397,12 @@ int dss2_mlp2_bwd_nh(int64_t num_nodes, const float* x, int din, const float* w1
 
 /* ------------------------------------------------------------------------------------------------
  * gnn_dsse building blocks (networks.py:11-69: GCN2Conv / TAGConv / FAConv stacks at width dim_feat <= 8 on the one-way edge list as given).
- * dss2_gcn_dinv: gcn_norm's deg^-1/2 per bus (in-degree, + 1 with add_self_loops; inf -> 0).
+ * self_loops != 0 is gcn_norm(add_self_loops=True), i.e. PyG's add_remaining_self_loops: the self loops of the input are dropped and
+ * one loop of weight 1 per bus is appended; self_loops == 0 takes the edge list as given (an input loop is an ordinary edge).
+ * dss2_gcn_dinv: gcn_norm's deg^-1/2 per bus (in-degree; with add_self_loops input loops not counted, + 1; inf -> 0).
  * dss2_gcn_prop8: out = scale * (A_hat x) + add_scale * add with A_hat = D^-1/2 (A [+ I]) D^-1/2 over the in-edges in PyG's scatter
- *   order (self loop last), or - transposed != 0 - over the out-edges (adjoint).  Rows are 8 floats (zero padded), x with row stride.
+ *   order (self loop last; with self_loops the input loops skipped), or - transposed != 0 - over the out-edges (adjoint).  Rows are
+ *   8 floats (zero padded), x with row stride.
  * dss2_lin8_fwd/bwd: y = act(sum_m in_m W_m [+ b]) per bus for M <= 4 inputs of width 8; weight_is_out_by_in = 1 for torch Linear
  *   weights [out, in] (TAGConv.lins), 0 for GCN2Conv.weight1 [in, out]; act: 0 none, 1 leaky_relu(slope), 2 relu, 3 tanh.  The backward
  *   writes grad_z, grad_in[m], optionally acc += acc_scale * grad_in[0], and per-CTA partial sums of the weight gradients (layout of w)
@@ -416,6 +419,7 @@ int dss2_lin8_bwd(int64_t num_nodes, int M, int weight_is_out_by_in, const float
 
 /* gnn_dsse(model='fagcn') (networks.py:44-50, torch_geometric FAConv; dropout: dss2_fa_fwd_drop below) at width 8 on the one-way edge list:
  *   y[i] = act( sum_{j -> i} tanh(att_l . x[j] + att_r . x[i]) dinv[j] dinv[i] x[j]  (+ self loop, last)  + eps x0[i] ).
+ * With self_loops the input loops are skipped and one loop per bus is appended (as dss2_gcn_prop8; dinv from dss2_gcn_dinv alike).
  * dss2_fa_bwd: grad_x (adjoint of x, message and attention paths), optionally acc_x0 += eps * grad_z (the x_0 path), and per-CTA
  * partial sums of the attention gradients at partials[0..8) (att_l) and partials[8..16) (att_r), dss2_num_partials() rows. */
 int dss2_fa_fwd(const dss2_graph_t* g, const float* dinv, int self_loops, const float* x, int64_t x_stride, const float* x0,
@@ -431,8 +435,9 @@ int dss2_fa_bwd(const dss2_graph_t* g, const float* dinv, int self_loops, const 
  * Descriptor (host struct, one per layer and head):
  *   p in [0, 1); mode 0 none, 1 counter-based Philox keyed by (seed, step) read from DEVICE memory rng_state[2] (graph-replay safe, as
  *   dss2_tag_fwd) with layer_uid and head, 2 caller mask `mask` (uint8 [Et + Nt], 1 = keep).  p == 0 or mode 0 = no dropout.
- *   Edge key of a coefficient: the one-way edge id e for a real edge, Et + i for the loop appended at bus i (mode 2: entries of
- *   dropped input self loops are ignored, the loop entries are unused without add_self_loops).
+ *   Edge key of a coefficient: the one-way edge id e for a real edge, Et + i for the loop appended at bus i.  With add_self_loops both
+ *   GATv2 and FAConv drop the input self loops, so their keys are never read (mode 2: their mask entries are ignored); without it an
+ *   input loop is an ordinary edge with its own key and the loop entries Et + i are unused.
  * The forward and both backward passes re-draw the same bit wherever they visit a coefficient; nothing is stored between them.
  * dss2_gat_fwd_drop / dss2_gat_bwd_drop: dss2_gat_fwd / dss2_gat_bwd_ex with a weight slot (slot >= 0: dss2_gat_upload's weights, the
  *   pointers are ignored; -1: weights from the pointers) and a descriptor (NULL = none).  bwd: part_off NULL = the standard partial row.

@@ -354,15 +354,18 @@ def init_gine_state_dict(dim_feat=8, dim_dense=32, dim_out=2, num_layers=8, edge
 
 
 def gcn_norm_self_loops(edge_index, num_nodes, dtype):
-    """PyG gcn_norm(add_self_loops=True) for an edge list without self loops: the edges keep their order, one loop per node is
-    appended; deg = in-degree + 1 by target; w = deg[src]^-1/2 * deg[dst]^-1/2."""
+    """PyG gcn_norm(add_self_loops=True), which calls add_remaining_self_loops: the self loops of the input are dropped, the other
+    edges keep their order and one loop of weight 1 per node is appended; deg = in-degree (input loops not counted) + 1 by target;
+    w = deg[src]^-1/2 * deg[dst]^-1/2."""
     loop = torch.arange(num_nodes)
-    ei = torch.cat([edge_index, torch.stack([loop, loop])], dim=1)
+    ei = torch.cat([edge_index[:, edge_index[0] != edge_index[1]], torch.stack([loop, loop])], dim=1)
     return ei, gcn_weights(ei, num_nodes, dtype)
 
 
-def gnn_dsse_forward(sd, x, edge_index, num_layers, model="gcn2", alpha=0.1, K=3, add_self_loops=True, slope=0.01):
-    """gnn_dsse.forward (networks.py:67-69) from a reference-named state_dict (`model.module_{2l}.weight1` / `.lins.{k}.weight`, `.bias`)."""
+def gnn_dsse_forward(sd, x, edge_index, num_layers, model="gcn2", alpha=0.1, K=3, add_self_loops=True, slope=0.01, nonlin="leaky_relu"):
+    """gnn_dsse.forward (networks.py:67-69) from a reference-named state_dict (`model.module_{2l}.weight1` / `.lins.{k}.weight`, `.bias`).
+    nonlin: the module's activation after every conv, 'leaky_relu' (negative slope `slope`), 'relu' or 'tanh'."""
+    act = {"leaky_relu": lambda t: torch.nn.functional.leaky_relu(t, slope), "relu": torch.relu, "tanh": torch.tanh}[nonlin]
     n = x.size(0)
     x0, h = x, x
     for l in range(num_layers - 1):
@@ -395,7 +398,7 @@ def gnn_dsse_forward(sd, x, edge_index, num_layers, model="gcn2", alpha=0.1, K=3
             h = tag_conv(h, edge_index, ws, sd.get(p + "bias"))
         else:
             raise NotImplementedError(model)
-        h = torch.nn.functional.leaky_relu(h, slope)
+        h = act(h)
     i = 2 * (num_layers - 1)
     h = h @ sd[f"model.module_{i}.weight"].t() + sd[f"model.module_{i}.bias"]
     return h @ sd[f"model.module_{i + 1}.weight"].t() + sd[f"model.module_{i + 1}.bias"]

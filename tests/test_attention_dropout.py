@@ -22,27 +22,26 @@ P = 0.3
 
 
 # ------------------------------------------------------------------------------------------------ masked reference
-def edge_keys(edge_index, n, self_loops, drop_input_loops=True):
+def edge_keys(edge_index, n, self_loops):
     """Edge key of every attention coefficient in PyG's edge order: with self loops, the input loops removed (GATv2Conv's
-    remove_self_loops; the fagcn oracle keeps them) and one loop per bus appended; without, the edge list as given."""
+    remove_self_loops, FAConv's add_remaining_self_loops) and one loop per bus appended; without, the edge list as given."""
     et = edge_index.size(1)
     ids = torch.arange(et)
     if not self_loops:
         return ids
-    if drop_input_loops:
-        ids = ids[edge_index[0] != edge_index[1]]
+    ids = ids[edge_index[0] != edge_index[1]]
     return torch.cat([ids, et + torch.arange(n)])
 
 
-def to_pyg_order(mask, edge_index, n, self_loops, drop_input_loops=True):
+def to_pyg_order(mask, edge_index, n, self_loops):
     """[..., Et + N] edge-key layout -> [..., E'] PyG order."""
-    return mask[..., edge_keys(edge_index, n, self_loops, drop_input_loops)]
+    return mask[..., edge_keys(edge_index, n, self_loops)]
 
 
-def from_pyg_order(mask, edge_index, n, self_loops, drop_input_loops=True):
+def from_pyg_order(mask, edge_index, n, self_loops):
     """[..., E'] PyG order -> [..., Et + N] edge-key layout (keys PyG never visits: 0)."""
     out = torch.zeros(mask.shape[:-1] + (edge_index.size(1) + n,), dtype=mask.dtype)
-    out[..., edge_keys(edge_index, n, self_loops, drop_input_loops)] = mask
+    out[..., edge_keys(edge_index, n, self_loops)] = mask
     return out
 
 
@@ -105,7 +104,7 @@ def fa_layer(h, x0, edge_index, att_l, att_r, eps, self_loops=True, mask=None, p
         ei, w = edge_index, orc.gcn_weights(edge_index, n, h.dtype)
     t = torch.tanh((h @ att_l.t())[ei[0]] + (h @ att_r.t())[ei[1]]).squeeze(-1)
     if mask is not None:
-        t = t * (to_pyg_order(mask, edge_index, n, self_loops, drop_input_loops=False).to(h.dtype) / (1.0 - p))
+        t = t * (to_pyg_order(mask, edge_index, n, self_loops).to(h.dtype) / (1.0 - p))
     out = orc.segment_sum((t * w).view(-1, 1) * h[ei[0]], ei[1], n)
     return out + eps * x0 if eps != 0.0 else out
 
@@ -179,17 +178,21 @@ def test_masked_gatv2_reference_matches_pyg_semantics(monkeypatch, heads, self_l
 
 @pytest.mark.parametrize("self_loops", [True, False])
 def test_masked_faconv_reference_matches_pyg_semantics(monkeypatch, self_loops):
+    """On the loop-free graph and on _EI, whose input loops FAConv's add_remaining_self_loops drops under add_self_loops (their mask
+    entries are then never read) and keeps as ordinary edges without it."""
     conv = _shim_conv()
     n = 9
     torch.manual_seed(12)
     x, x0 = torch.randn(n, 8, dtype=torch.float64), torch.randn(n, 8, dtype=torch.float64)
     layer = conv.FAConv(8, eps=0.1, dropout=P, add_self_loops=self_loops).double().train()
-    mask = random_masks(2, 1, _EI_NO_LOOPS.size(1) + n, P, seed=5)[0][0]
-    mask_pyg = to_pyg_order(mask, _EI_NO_LOOPS, n, self_loops, drop_input_loops=False)
-    _patched_dropout(monkeypatch, mask_pyg)
-    want = layer(x, x0, _EI_NO_LOOPS)
-    got = fa_layer(x, x0, _EI_NO_LOOPS, layer.att_l.weight.detach(), layer.att_r.weight.detach(), 0.1, self_loops, mask, P)
-    assert torch.allclose(got, want, rtol=1e-12, atol=1e-12)
+    for ei in (_EI_NO_LOOPS, _EI):
+        mask = random_masks(2, 1, ei.size(1) + n, P, seed=5)[0][0]
+        mask_pyg = to_pyg_order(mask, ei, n, self_loops)
+        _patched_dropout(monkeypatch, mask_pyg)
+        want = layer(x, x0, ei)
+        monkeypatch.undo()
+        got = fa_layer(x, x0, ei, layer.att_l.weight.detach(), layer.att_r.weight.detach(), 0.1, self_loops, mask, P)
+        assert torch.allclose(got, want, rtol=1e-12, atol=1e-12)
 
 
 def test_constructors_accept_attention_dropout(monkeypatch):
