@@ -45,3 +45,12 @@ extern "C" int dss2_adamax_step(float* param, const float* grad, float* exp_avg,
   }
   return 0;
 }
+
+// The clock of a forward-only stream (the captured evaluator): one increment per forward keeps its dropout draws and tile-mark
+// sequence numbers fresh on every replay.
+extern "C" int dss2_step_advance(uint64_t* step_state, void* stream_) {
+  DSS2_CHECK_ARG(step_state, "dss2_step_advance: null argument");
+  k_bump<<<1, 1, 0, (cudaStream_t)stream_>>>(step_state);
+  DSS2_LAUNCH_CHECK();
+  return 0;
+}

@@ -511,17 +511,33 @@ int wls_generic(const WlsArgs& a, bool want_grad, cudaStream_t stream) {
 }
 
 // get_pflow as a plain per-branch kernel (evaluation path, dss2_run.py:193-194): outputs are API tensors.
-__global__ void k_pflow(const int64_t* __restrict__ ei, int64_t Et, const float* __restrict__ y, int64_t ys,
+// EST: y is the model output (normalised V, raw theta) and the bus state is the de-normalised estimate of dss2_run.py:183-184,
+// V = y0 * x_std0 + x_mean0 and theta = y1 * (1 - x[:, 9]) - the arithmetic of k_eval_metrics' estimate branch.
+struct PflowEst {
+  const float* x;   // [Nt, >= 10]: column 9 = slack flag
+  int64_t xs;
+  float xm0, xs0;
+};
+template <bool EST>
+__device__ __forceinline__ void pflow_bus(const float* y, int64_t ys, const PflowEst& est, int64_t n, float& v, float& th) {
+  if (EST) {
+    v = y[n * ys] * est.xs0 + est.xm0;
+    th = y[n * ys + 1] * (1.0f - est.x[n * est.xs + 9]);
+  } else {
+    v = y[n * ys];
+    th = y[n * ys + 1];
+  }
+}
+template <bool EST>
+__global__ void k_pflow(const int64_t* __restrict__ ei, int64_t Et, const float* __restrict__ y, int64_t ys, PflowEst est,
                         const float* __restrict__ ep, int64_t eps_, const float* __restrict__ vminmax, float* out8, int use_shift) {
   const WlsGrid grid = wls_grid(vminmax[0], vminmax[1]);
   for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < Et; e += (int64_t)gridDim.x * blockDim.x) {
     int64_t i = ei[e], j = ei[Et + e];
     const float* row = ep + e * eps_;
     WlsBranchIn in;
-    in.vi = y[i * ys];
-    in.thi = y[i * ys + 1];
-    in.vj = y[j * ys];
-    in.thj = y[j * ys + 1];
+    pflow_bus<EST>(y, ys, est, i, in.vi, in.thi);
+    pflow_bus<EST>(y, ys, est, j, in.vj, in.thj);
     in.G = row[0];
     in.B = row[1];
     in.Gs = row[2];
@@ -604,10 +620,37 @@ struct EvalArgs {
   const float* vminmax;
   double* partial;     // [grid][M_N]
   unsigned* counter;
-  double* sums;        // [M_N]
+  double* sums;        // [M_N] or NULL
+  double* acc;         // [EVAL_ACC_N] or NULL: the batch's finalised metrics are added here (eval_finalise)
 };
+
+// The ten metrics of one batch from its 19 sums, in the order of dss2.metrics.evaluate_batch's dict, exactly as the script's formulas
+// compute them in fp64 (wls.o is built with -fmad=false; double sqrt and division are IEEE): the epoch accumulator gets each value
+// added, and one more batch counted in [10].  Python semantics kept where CUDA's differ: ratio(a, 0) = NaN, the std of n <= 1 values is
+// NaN, and max(v, 0.0) keeps a NaN v (fmax would return 0).
+enum { EVAL_ACC_N = 11 };
+__device__ __forceinline__ double eval_nan() { return __longlong_as_double(0x7ff8000000000000LL); }   // Python's float("nan")
+__device__ __forceinline__ double eval_ratio(double a, double b) { return b != 0.0 ? a / b : eval_nan(); }
+__device__ __forceinline__ double eval_std(double sx, double sxx, double n) {   // torch.std: unbiased
+  if (!(n > 1.0)) return eval_nan();
+  const double v = (sxx - sx * sx / n) / (n - 1.0);
+  return sqrt(0.0 > v ? 0.0 : v);
+}
+__device__ void eval_finalise(const double* s, double n, double* acc) {
+  const double m[10] = {
+      sqrt(s[M_SE_V] / n), s[M_AE_V] / n, sqrt(s[M_SE_TH] / n), s[M_AE_TH] / n,
+      sqrt(eval_ratio(s[M_SE_L], s[M_CNT_L])), eval_ratio(s[M_AE_L], s[M_CNT_L]),
+      sqrt(eval_ratio(s[M_SE_T], s[M_CNT_T])), eval_ratio(s[M_AE_T], s[M_CNT_T]),
+      100.0 * eval_ratio(eval_std(s[M_SV], s[M_SVV], n), eval_std(s[M_YV], s[M_YVV], n)),
+      100.0 * eval_ratio(eval_std(s[M_STH], s[M_STHTH], n), eval_std(s[M_YTH], s[M_YTHTH], n))};
+#pragma unroll
+  for (int k = 0; k < 10; ++k) acc[k] += m[k];
+  acc[10] += 1.0;
+}
+
 __global__ void __launch_bounds__(WLS_THREADS) k_eval_metrics(EvalArgs a) {
   __shared__ double s_red[M_N][WLS_THREADS / 32];
+  __shared__ double s_tot[M_N];
   __shared__ bool s_last;
   const WlsGrid grid = wls_grid(a.vminmax[0], a.vminmax[1]);
   double acc[M_N];
@@ -688,9 +731,16 @@ __global__ void __launch_bounds__(WLS_THREADS) k_eval_metrics(EvalArgs a) {
       double v = 0;
       for (unsigned c = lane; c < gridDim.x; c += 32) v += ((volatile double*)a.partial)[(size_t)c * M_N + q];
       v = warp_sum(v);
-      if (lane == 0) a.sums[q] = v;
+      if (lane == 0) {
+        if (a.sums) a.sums[q] = v;
+        s_tot[q] = v;
+      }
     }
     if (tid == 0) *a.counter = 0;
+    if (a.acc) {          // s_last is uniform over the CTA
+      __syncthreads();
+      if (tid == 0) eval_finalise(s_tot, (double)a.Nt, a.acc);
+    }
   }
 }
 
@@ -783,14 +833,16 @@ static int wls_launch(int phase, const dss2_graph_t* g, const float* x, int64_t 
 
 extern "C" size_t dss2_eval_workspace_bytes(void) { return 256 + (size_t)(dss2_sm_count() * 4 + 1) * M_N * sizeof(double); }
 
-extern "C" int dss2_eval_metrics(const int64_t* edge_index, int64_t num_nodes, int64_t num_edges, const float* x, int64_t x_stride,
-                                 const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y,
-                                 int64_t y_stride, float x_mean0, float x_std0, const float* vminmax, double* sums19, void* ws,
-                                 size_t ws_bytes, void* stream_) {
+// sums19 and acc11: exactly one of them is set (dss2_eval_metrics / dss2_eval_metrics_acc)
+static int eval_launch(const int64_t* edge_index, int64_t num_nodes, int64_t num_edges, const float* x, int64_t x_stride,
+                       const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y, int64_t y_stride,
+                       float x_mean0, float x_std0, const float* vminmax, double* sums19, double* acc11, void* ws, size_t ws_bytes,
+                       void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
-  DSS2_CHECK_ARG(edge_index && x && edge_attr && output && y && vminmax && sums19 && ws, "dss2_eval_metrics: null argument");
-  DSS2_CHECK_ARG(x_stride >= 11 && ea_stride >= 13 && out_stride >= 2 && y_stride >= 2, "dss2_eval_metrics: x needs 11 columns, edge_attr 13");
-  DSS2_CHECK_ARG(ws_bytes >= dss2_eval_workspace_bytes(), "dss2_eval_metrics: workspace too small");
+  const char* who = acc11 ? "dss2_eval_metrics_acc" : "dss2_eval_metrics";
+  DSS2_CHECK_ARG(edge_index && x && edge_attr && output && y && vminmax && (sums19 || acc11) && ws, "%s: null argument", who);
+  DSS2_CHECK_ARG(x_stride >= 11 && ea_stride >= 13 && out_stride >= 2 && y_stride >= 2, "%s: x needs 11 columns, edge_attr 13", who);
+  DSS2_CHECK_ARG(ws_bytes >= dss2_eval_workspace_bytes(), "%s: workspace too small", who);
   EvalArgs a;
   a.Nt = num_nodes;
   a.Et = num_edges;
@@ -809,10 +861,29 @@ extern "C" int dss2_eval_metrics(const int64_t* edge_index, int64_t num_nodes, i
   a.counter = (unsigned*)ws;                      // zero-initialised by the caller once; self-resetting
   a.partial = (double*)((char*)ws + 256);
   a.sums = sums19;
+  a.acc = acc11;
   const int grid = (int)max((int64_t)1, min((int64_t)dss2_sm_count() * 4, (max(num_nodes, num_edges) + WLS_THREADS - 1) / WLS_THREADS));
   k_eval_metrics<<<grid, WLS_THREADS, 0, stream>>>(a);
   DSS2_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int dss2_eval_metrics(const int64_t* edge_index, int64_t num_nodes, int64_t num_edges, const float* x, int64_t x_stride,
+                                 const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y,
+                                 int64_t y_stride, float x_mean0, float x_std0, const float* vminmax, double* sums19, void* ws,
+                                 size_t ws_bytes, void* stream_) {
+  DSS2_CHECK_ARG(sums19, "dss2_eval_metrics: null argument");
+  return eval_launch(edge_index, num_nodes, num_edges, x, x_stride, edge_attr, ea_stride, output, out_stride, y, y_stride, x_mean0, x_std0,
+                     vminmax, sums19, nullptr, ws, ws_bytes, stream_);
+}
+
+extern "C" int dss2_eval_metrics_acc(const int64_t* edge_index, int64_t num_nodes, int64_t num_edges, const float* x, int64_t x_stride,
+                                     const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y,
+                                     int64_t y_stride, float x_mean0, float x_std0, const float* vminmax, double* acc11, void* ws,
+                                     size_t ws_bytes, void* stream_) {
+  DSS2_CHECK_ARG(acc11, "dss2_eval_metrics_acc: null argument");
+  return eval_launch(edge_index, num_nodes, num_edges, x, x_stride, edge_attr, ea_stride, output, out_stride, y, y_stride, x_mean0, x_std0,
+                     vminmax, nullptr, acc11, ws, ws_bytes, stream_);
 }
 
 extern "C" int dss2_pflow(const int64_t* edge_index, int64_t Et, const float* y, int64_t y_stride, const float* edge_param,
@@ -820,13 +891,27 @@ extern "C" int dss2_pflow(const int64_t* edge_index, int64_t Et, const float* y,
   return dss2_pflow_ex(edge_index, Et, y, y_stride, edge_param, ep_stride, vminmax, 0, out8, stream_);
 }
 
+static int pflow_grid(int64_t Et) { return (int)max((int64_t)1, min((int64_t)148 * 8, (Et + 255) / 256)); }
+
 extern "C" int dss2_pflow_ex(const int64_t* edge_index, int64_t Et, const float* y, int64_t y_stride, const float* edge_param,
                              int64_t ep_stride, const float* vminmax, int use_shift, float* out8, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   DSS2_CHECK_ARG(edge_index && y && edge_param && vminmax && out8, "dss2_pflow: null argument");
   if (Et == 0) return 0;
-  int grid = (int)max((int64_t)1, min((int64_t)148 * 8, (Et + 255) / 256));
-  k_pflow<<<grid, 256, 0, stream>>>(edge_index, Et, y, y_stride, edge_param, ep_stride, vminmax, out8, use_shift);
+  k_pflow<false><<<pflow_grid(Et), 256, 0, stream>>>(edge_index, Et, y, y_stride, PflowEst{}, edge_param, ep_stride, vminmax, out8, use_shift);
+  DSS2_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int dss2_pflow_est(const int64_t* edge_index, int64_t Et, const float* output, int64_t out_stride, const float* x, int64_t x_stride,
+                              float x_mean0, float x_std0, const float* edge_param, int64_t ep_stride, const float* vminmax, float* out8,
+                              void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  DSS2_CHECK_ARG(edge_index && output && x && edge_param && vminmax && out8, "dss2_pflow_est: null argument");
+  DSS2_CHECK_ARG(out_stride >= 2 && x_stride >= 10, "dss2_pflow_est: output needs 2 columns, x 10");
+  if (Et == 0) return 0;
+  k_pflow<true><<<pflow_grid(Et), 256, 0, stream>>>(edge_index, Et, output, out_stride, PflowEst{x, x_stride, x_mean0, x_std0}, edge_param,
+                                                    ep_stride, vminmax, out8, 0);
   DSS2_LAUNCH_CHECK();
   return 0;
 }

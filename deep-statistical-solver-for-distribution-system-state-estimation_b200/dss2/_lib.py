@@ -79,10 +79,14 @@ _SIGNATURES = {
     "dss2_pflow": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, _P, _P]),
     "dss2_pflow_ex": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, c_int, _P, _P]),
     "dss2_pflow_bwd": (c_int, [_G, _P, c_int64, _P, c_int64, _P, c_int, _P, _P, _P]),
+    "dss2_pflow_est": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, c_float, c_float, _P, c_int64, _P, _P, _P]),
     "dss2_adamax_step": (c_int, [_P, _P, _P, _P, c_int64, c_float, c_float, c_float, c_float, c_float, _P, c_int, _P]),
+    "dss2_step_advance": (c_int, [_P, _P]),
     "dss2_eval_workspace_bytes": (c_size_t, []),
     "dss2_eval_metrics": (c_int, [_P, c_int64, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, c_float, c_float, _P, _P, _P,
                                   c_size_t, _P]),
+    "dss2_eval_metrics_acc": (c_int, [_P, c_int64, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, _P, c_int64, c_float, c_float, _P, _P,
+                                      _P, c_size_t, _P]),
     "dss2_gat_ws_bytes": (c_size_t, [c_int64]),
     "dss2_gat_fwd": (c_int, [_G, _P, c_int64, _P, c_int64, c_int, _P, _P, _P, _P, _P, _P, _P, c_float, c_int, c_float, _P, _P]),
     "dss2_gat_bwd": (c_int, [_G, _P, c_int64, _P, c_int64, c_int, _P, _P, _P, _P, _P, _P, _P, c_float, c_int, c_float,

@@ -1,13 +1,26 @@
 """Validation metrics of the reference script on the device (SURVEY.md 8f-4): one kernel per batch instead of the ~40 eager ops,
-two `get_pflow` calls, `nonzero()` filtering and torchmetrics objects of dss2_run.py:183-209."""
-import math
-
+two `get_pflow` calls, `nonzero()` filtering and torchmetrics objects of dss2_run.py:183-209.  The metric formulas live in that kernel's
+finaliser (csrc/wls.cu, `dss2_eval_metrics_acc`), which both this module and the captured evaluator (dss2.evaluator) read."""
 import torch
 
 from . import _lib
 from .ops import require_cuda, stage_rows
 
 _WS = {}
+
+# the ten metrics of one batch, in the order of the finaliser's accumulator (acc11[0..9]; acc11[10] counts the batches)
+KEYS = ("rmse_v", "mae_v", "rmse_th", "mae_th", "rmse_loading", "mae_loading", "rmse_loading_trafos", "mae_loading_trafos",
+        "prop_std_v", "prop_std_th")
+
+
+def epoch_means(acc):
+    """Host dict of an fp64 accumulator [11]: acc[k] / acc[10] per metric (the script's mean over batches) and "batches".
+    One device-to-host copy."""
+    a = acc.cpu().tolist()
+    nb = a[10]
+    res = {k: (a[i] / nb if nb else float("nan")) for i, k in enumerate(KEYS)}
+    res["batches"] = int(nb)
+    return res
 
 
 def evaluate_batch(out, y, x, edge_index, edge_attr, x_mean, x_std):
@@ -31,22 +44,10 @@ def evaluate_batch(out, y, x, edge_index, edge_attr, x_mean, x_std):
             ws = _WS[dev.index] = torch.zeros(lib.dss2_eval_workspace_bytes(), dtype=torch.uint8, device=dev)
         vmm = torch.empty(2, dtype=torch.float32, device=dev)
         _lib.check(lib.dss2_col_minmax(_lib.ptr(xg), xs, 8, xg.size(0), _lib.ptr(vmm), _lib.stream()), "dss2_col_minmax")
-        sums = torch.empty(19, dtype=torch.float64, device=dev)
-        _lib.check(lib.dss2_eval_metrics(_lib.ptr(ei), xg.size(0), ei.size(1), _lib.ptr(xg), xs, _lib.ptr(eg), es, _lib.ptr(og), os_,
-                                         _lib.ptr(yg), ys, float(x_mean[0]), float(x_std[0]), _lib.ptr(vmm), _lib.ptr(sums),
-                                         _lib.ptr(ws), ws.numel(), _lib.stream()), "dss2_eval_metrics")
-    s = sums.cpu().tolist()
-    n = float(xg.size(0))
-
-    def std(sx, sxx):   # torch.std: unbiased
-        return math.sqrt(max((sxx - sx * sx / n) / (n - 1.0), 0.0)) if n > 1 else float("nan")
-
-    def ratio(a, b):
-        return a / b if b != 0.0 else float("nan")
-
-    return {
-        "rmse_v": math.sqrt(s[0] / n), "mae_v": s[1] / n, "rmse_th": math.sqrt(s[2] / n), "mae_th": s[3] / n,
-        "rmse_loading": math.sqrt(ratio(s[13], s[12])), "mae_loading": ratio(s[14], s[12]),
-        "rmse_loading_trafos": math.sqrt(ratio(s[16], s[15])), "mae_loading_trafos": ratio(s[17], s[15]),
-        "prop_std_v": 100.0 * ratio(std(s[4], s[5]), std(s[8], s[9])), "prop_std_th": 100.0 * ratio(std(s[6], s[7]), std(s[10], s[11])),
-    }
+        acc = torch.zeros(11, dtype=torch.float64, device=dev)     # one batch: its values / 1
+        _lib.check(lib.dss2_eval_metrics_acc(_lib.ptr(ei), xg.size(0), ei.size(1), _lib.ptr(xg), xs, _lib.ptr(eg), es, _lib.ptr(og), os_,
+                                             _lib.ptr(yg), ys, float(x_mean[0]), float(x_std[0]), _lib.ptr(vmm), _lib.ptr(acc),
+                                             _lib.ptr(ws), ws.numel(), _lib.stream()), "dss2_eval_metrics_acc")
+        res = epoch_means(acc)
+    del res["batches"]
+    return res

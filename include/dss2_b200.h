@@ -264,6 +264,12 @@ int dss2_pflow_ex(const int64_t* edge_index, int64_t num_edges, const float* y, 
                   int64_t ep_stride, const float* vminmax, int use_shift, float* out8, void* stream);
 int dss2_pflow_bwd(const dss2_graph_t* g, const float* y, int64_t y_stride, const float* edge_param, int64_t ep_stride,
                    const float* vminmax, int use_shift, const float* grad_out8, float* grad_y, void* stream);
+/* dss2_pflow_est: get_pflow of the model's de-normalised estimate (inference, dss2_run.py:183-194) without materialising it: per bus
+ * V = output[:,0] * x_std0 + x_mean0 and theta = output[:,1] * (1 - x[:,9]) (separately rounded fp32, as the torch ops compute it),
+ * then the branch flows of dss2_pflow into the same out8 [8,Et] layout.  output [Nt,>=2] (row stride out_stride), x [Nt,>=10]
+ * (x_stride); x_mean0 / x_std0 by value.  No host reads, no allocation: graph-capturable. */
+int dss2_pflow_est(const int64_t* edge_index, int64_t num_edges, const float* output, int64_t out_stride, const float* x, int64_t x_stride,
+                   float x_mean0, float x_std0, const float* edge_param, int64_t ep_stride, const float* vminmax, float* out8, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * (f-3) Dataset builder.  Replaces the feature engineering of data_from_pickles (data.py:96-206) for S scenarios of one grid:
@@ -301,6 +307,15 @@ int dss2_eval_metrics(const int64_t* edge_index, int64_t num_nodes, int64_t num_
                       const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y,
                       int64_t y_stride, float x_mean0, float x_std0, const float* vminmax, double* sums19, void* ws, size_t ws_bytes,
                       void* stream);
+/* Same kernel and arguments, with the batch finalised on the device for an epoch average that needs no host synchronisation: the last
+ * CTA turns the 19 sums into the ten metrics of dss2.metrics.evaluate_batch in fp64 (rmse_v, mae_v, rmse_th, mae_th, rmse_loading,
+ * mae_loading, rmse_loading_trafos, mae_loading_trafos, prop_std_v, prop_std_th; the script's formulas in its operation order, NaN where
+ * a count is zero or a std has n <= 1) and ADDS them to acc11[0..9], and 1 to acc11[10] (the batch count).  Epoch value k =
+ * acc11[k] / acc11[10], the script's mean over batches (dss2_run.py:165-236).  acc11: device fp64, zeroed by the caller per epoch. */
+int dss2_eval_metrics_acc(const int64_t* edge_index, int64_t num_nodes, int64_t num_edges, const float* x, int64_t x_stride,
+                          const float* edge_attr, int64_t ea_stride, const float* output, int64_t out_stride, const float* y,
+                          int64_t y_stride, float x_mean0, float x_std0, const float* vminmax, double* acc11, void* ws, size_t ws_bytes,
+                          void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Adjacent: flat-buffer Adamax (torch.optim.Adamax defaults, dss2_run.py:91-92,143).
@@ -311,6 +326,9 @@ int dss2_eval_metrics(const int64_t* edge_index, int64_t num_nodes, int64_t num_
 int dss2_adamax_step(float* param, const float* grad, float* exp_avg, float* exp_inf, int64_t count,
                      float lr, float beta1, float beta2, float eps, float grad_scale,
                      uint64_t* step_state, int bump, void* stream);
+/* step_state[1] += 1 on the device: the clock of a forward-only stream (a captured evaluator advances it once per forward, so that its
+ * dropout draws and the tile-mark sequence numbers of the chained layers differ on every replay). */
+int dss2_step_advance(uint64_t* step_state, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Next row (SURVEY.md 8f-1): GAT_DSSE, the as-shipped default model of dss2_run.py:86 (networks.py:113-156):
