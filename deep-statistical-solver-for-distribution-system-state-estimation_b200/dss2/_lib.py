@@ -33,9 +33,21 @@ class AttnDrop(Structure):
     _fields_ = [("p", c_float), ("mode", c_int), ("rng_state", c_void_p), ("layer_uid", c_uint32), ("head", c_uint32), ("mask", c_void_p)]
 
 
+class PfTopology(Structure):
+    """Mirror of `dss2_pf_topology_t` (one power-flow topology, dss2.powerflow)."""
+    _fields_ = [
+        ("num_buses", c_int32), ("slack", c_int32), ("num_pq", c_int32), ("num_blocks", c_int32),
+        ("num_updates", c_int32), ("num_edges", c_int32), ("v_lv", ctypes.c_double),
+        ("y_ptr", c_void_p), ("y_col", c_void_p), ("y_gb", c_void_p), ("bus", c_void_p), ("blk_ptr", c_void_p),
+        ("blk_col", c_void_p), ("blk_y", c_void_p), ("diag", c_void_p), ("upd_ptr", c_void_p), ("upd", c_void_p),
+        ("edge_ft", c_void_p), ("edge_gb", c_void_p),
+    ]
+
+
 _P = c_void_p
 _G = POINTER(GraphStruct)
 _D = POINTER(AttnDrop)
+_T = POINTER(PfTopology)
 _SIGNATURES = {
     "dss2_last_error": (c_char_p, []),
     "dss2_version": (c_int, []),
@@ -76,6 +88,9 @@ _SIGNATURES = {
     "dss2_build_scenarios": (c_int, [_P, _P, _P, _P, _P, _P, _P, c_int64, c_int, c_int, _P, _P, _P, _P, c_size_t, _P]),
     "dss2_load_profiles": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, ctypes.c_double, _P, _P, _P]),
     "dss2_mc_sample": (c_int, [_P, _P, c_int64, c_int, c_int, _P, _P, _P]),
+    "dss2_powerflow_workspace_bytes": (c_size_t, [_T, c_int64]),
+    "dss2_powerflow": (c_int, [_T, c_int64, _P, _P, _P, ctypes.c_double, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t,
+                               c_int64, _P]),
     "dss2_pflow": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, _P, _P]),
     "dss2_pflow_ex": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, c_int, _P, _P]),
     "dss2_pflow_bwd": (c_int, [_G, _P, c_int64, _P, c_int64, _P, c_int, _P, _P, _P]),

@@ -1,7 +1,8 @@
 """Synthetic scenario sampler of the reference's offline generator (scope row 8f-3): the 24-hour load / generation profiles and the
 Monte-Carlo perturbation of `toy_network.py:83-126` with the samplers of `loadsampling.py:75-107`, evaluated by two CUDA kernels
 (`dss2_load_profiles`, `dss2_mc_sample`, csrc/dataset.cu).  The power-flow solve that turns the sampled loads into labels (pandapower
-`runpp`, toy_network.py:160-250) is the reference's offline L0 stage and stays out of scope.
+`runpp`, toy_network.py:160-250) is `dss2.powerflow` (the reference's pi-model, on the device): sum the samples into bus injections and
+call `powerflow.solved_scenarios` (INTEGRATION.md 2).
 
 Random draws: by default they are taken from numpy's legacy global stream exactly like the reference's `np.random.rand` /
 `np.random.normal` calls (row-major over the Monte-Carlo matrix), so after `np.random.seed(s)` the samples equal the reference's bit for

@@ -296,6 +296,54 @@ int dss2_load_profiles(const double* base, const double* weight_a, const double*
 int dss2_mc_sample(const double* arg_a, const double* arg_b, int64_t U, int iters, int dist, const double* draws, double* out,
                    void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * (f-2) AC power flow of the offline generator.  Replaces pandapower runpp (toy_network.py:180, in the loop of :160-250) on the
+ * reference's own pi-model (data.py:370-376, phase shift ignored): Y_ff, Y_tt += y + ys/2 and Y_ft, Y_tf -= y per closed edge, parallel
+ * edges summed; S_calc = V_lv^2 U conj(Y U), V_lv = min(vn_kv); S_spec = -(p_mw + j q_mvar) (load-positive, data.py:428-429).
+ * Newton-Raphson in polar form, fp64, from a flat start (V = 1, theta = 0; the slack at (v_slack[s], 0)); one slack bus, PQ buses.
+ * Topology (built once on the host, dss2.powerflow.symbolic; every array DEVICE, int32 unless stated):
+ *   y_ptr [N+1], y_col, y_gb [nnz,2] f64: Y * V_lv^2 as CSR over all buses (MVA at 1 pu);
+ *   bus [n]: bus of elimination position k (n = N - 1, the slack removed);
+ *   blk_ptr [n+1], blk_col [blocks]: 2x2-block pattern of the reduced Jacobian in position order with fill, columns ascending;
+ *   blk_y [blocks]: Y entry of each block (-1 = fill); diag [n]: position of block (k,k);
+ *   upd_ptr [blocks+1], upd [updates,2]: for lower block p = (k,m), the pairs (block (k,j), block (m,j)), j > m, of the row-wise block LU;
+ *   edge_ft [E,2], edge_gb [E,4] f64 (G, B, Gs, Bs): the closed edges, whose flows are returned.
+ * dss2_powerflow: p_mw, q_mvar [S,N] (slack entries ignored), v_slack [S].  Per scenario, convergence (max |S_calc - S_spec| over the PQ
+ *   buses <= tol_mva) is tested before each update; iterations [S] = updates applied.  Out: vm_pu, va_rad [S,N]; p_out, q_out [S,N] get
+ *   the slack's computed injection at the slack column (other entries untouched: the caller copies the inputs in); p_from, q_from,
+ *   p_to, q_to [S,E] (rounded like synth.branch_flows); converged [S] u8; max_mismatch [S] (MVA, at the last evaluation).  max_iter
+ *   updates without convergence, or a pivot with |det| <= 1e-12 (|ad| + |bc|), give converged = 0 and undefined outputs for that
+ *   scenario only.  Scenarios run `chunk` per launch in `workspace` (dss2_powerflow_workspace_bytes(topo, chunk) = 8 chunk (4 N + 2 n +
+ *   4 blocks) bytes); no atomics, so a scenario's result does not depend on the chunk or the other scenarios.  No host synchronisation,
+ *   no allocation.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dss2_pf_topology {
+  int32_t num_buses;        /* N */
+  int32_t slack;
+  int32_t num_pq;           /* n = N - 1 */
+  int32_t num_blocks;
+  int32_t num_updates;
+  int32_t num_edges;        /* E closed edges */
+  double v_lv;              /* min(vn_kv), kV */
+  const int32_t* y_ptr;
+  const int32_t* y_col;
+  const double* y_gb;
+  const int32_t* bus;
+  const int32_t* blk_ptr;
+  const int32_t* blk_col;
+  const int32_t* blk_y;
+  const int32_t* diag;
+  const int32_t* upd_ptr;
+  const int32_t* upd;
+  const int32_t* edge_ft;
+  const double* edge_gb;
+} dss2_pf_topology_t;
+size_t dss2_powerflow_workspace_bytes(const dss2_pf_topology_t* topo, int64_t chunk);
+int dss2_powerflow(const dss2_pf_topology_t* topo, int64_t S, const double* p_mw, const double* q_mvar, const double* v_slack,
+                   double tol_mva, int max_iter, double* vm_pu, double* va_rad, double* p_out, double* q_out, double* p_from,
+                   double* q_from, double* p_to, double* q_to, int32_t* iterations, uint8_t* converged, double* max_mismatch,
+                   void* workspace, size_t workspace_bytes, int64_t chunk, void* stream);
+
 /* Validation metrics of one batch (SURVEY.md 8f-4, dss2_run.py:183-209) in one kernel: x [Nt,>=11] (column 9 = slack flag),
  * edge_attr [Et,>=13] (columns 6.. = branch parameters), output [Nt,2] = model output (normalised V, raw theta), y [Nt,2] = labels.
  * sums19 (device, fp64): [0..3] sum (dV)^2, |dV|, (dth)^2, |dth| with V = out0*x_std0 + x_mean0 and th = out1*(1-slack);
