@@ -176,7 +176,75 @@ __global__ void k_build_ell(dss2_graph_t g) {
       cols |= (uint32_t)(local & 0xff) << (8 * d);
     }
     reinterpret_cast<float4*>(g.ell_w)[n] = make_float4(w[0], w[1], w[2], w[3]);
-    reinterpret_cast<uint2*>(g.ell_ci)[n] = make_uint2(cols, (uint32_t)deg);
+    reinterpret_cast<uint2*>(g.ell_ci)[n] = make_uint2(cols, (uint32_t)min(deg, (int)DSS2_ELL_DEG_MASK));
+  }
+}
+
+// Swizzle keys of one tile's rows (see DSS2_HOP_KEYS_COLOR in dss2_b200.h).  ci = the tile's ELL words before key packing, key = out.
+// The 8 lanes of one LDS.128 / STS.128 phase of the layer kernels are 8 consecutive tile rows (group G = rows 8j..8j+7), each
+// reading or writing 16 bytes of one row of the plain level tile; two of them hit the same banks iff their rows differ and have the
+// same key.  Costs, per pair of distinct rows with equal keys:
+//   (a) 4 for the slot-d sources of two rows of one group (gathered together: up to 4 slots x 4 loads per thread and hop),
+//   (b) 1 for two rows of one group (stored together: 4 stores per thread and level).
+// Greedy colouring in row order, then two sweeps that move each row to its cheapest key (more sweeps change nothing on the grids
+// in the repository); ties keep the identity key (n0 + r) & 7.  Deterministic: integer costs, fixed order.
+__host__ __device__ void hop_keys_tile(const uint2* ci, int nT, int n0, int policy, uint8_t* key) {
+  constexpr int WA = 4, WB = 1, NO_KEY = 0xff;
+  if (policy != DSS2_HOP_KEYS_COLOR) {
+    for (int r = 0; r < nT; ++r) key[r] = (uint8_t)((n0 + r) & 7);
+    return;
+  }
+  uint16_t start[DSS2_TILE_CAP + 1], occ[4 * DSS2_TILE_CAP];   // (row, slot) pairs grouped by source row
+  for (int v = 0; v <= nT; ++v) start[v] = 0;
+  auto active = [&](int r) { return (int)min(ci[r].y & DSS2_ELL_DEG_MASK, 4u); };
+  auto src = [&](int r, int d) { return (int)((ci[r].x >> (8 * d)) & 0xffu); };
+  for (int r = 0; r < nT; ++r)
+    for (int d = 0; d < active(r); ++d) ++start[src(r, d) + 1];
+  for (int v = 0; v < nT; ++v) start[v + 1] += start[v];
+  {
+    uint16_t fill[DSS2_TILE_CAP];
+    for (int v = 0; v < nT; ++v) fill[v] = start[v];
+    for (int r = 0; r < nT; ++r)
+      for (int d = 0; d < active(r); ++d) occ[fill[src(r, d)]++] = (uint16_t)(4 * r + d);
+  }
+  for (int r = 0; r < nT; ++r) key[r] = NO_KEY;
+  for (int pass = 0; pass < 3; ++pass) {
+    for (int v = 0; v < nT; ++v) {
+      int cost[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+      const int g0 = v & ~7, g1 = min(g0 + 8, nT);
+      for (int u = g0; u < g1; ++u)
+        if (u != v && key[u] != NO_KEY) cost[key[u]] += WB;
+      for (int o = start[v]; o < start[v + 1]; ++o) {
+        const int r = occ[o] >> 2, d = occ[o] & 3, h0 = r & ~7, h1 = min(h0 + 8, nT);
+        for (int q = h0; q < h1; ++q) {
+          if (q == r || d >= active(q)) continue;
+          const int s = src(q, d);
+          if (s != v && key[s] != NO_KEY) cost[key[s]] += WA;
+        }
+      }
+      int best = key[v] != NO_KEY ? key[v] : (n0 + v) & 7;   // ties keep the current (first pass: identity) key
+      for (int k = 0; k < 8; ++k)
+        if (cost[k] < cost[best]) best = k;
+      key[v] = (uint8_t)best;
+    }
+  }
+}
+
+// one thread per tile: keys -> hop_key[] and the upper bits of the tile's ELL degree words
+__global__ void k_hop_keys(dss2_graph_t g, int policy) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= g.num_tiles) return;
+  const TileRange r = tile_range(g, t);
+  const int nT = r.n1 - r.n0;
+  uint2* ci = reinterpret_cast<uint2*>(g.ell_ci) + r.n0;
+  uint8_t* key = g.hop_key + r.n0;
+  hop_keys_tile(ci, nT, r.n0, policy, key);
+  for (int i = 0; i < nT; ++i) {
+    const uint2 c = ci[i];
+    uint32_t word = (c.y & DSS2_ELL_DEG_MASK) | ((uint32_t)key[i] << DSS2_ELL_KEY_SHIFT);
+    const int act = (int)min(c.y & DSS2_ELL_DEG_MASK, 4u);
+    for (int d = 0; d < act; ++d) word |= (uint32_t)key[(c.x >> (8 * d)) & 0xffu] << (DSS2_ELL_KEY_SHIFT + 3 + 3 * d);
+    ci[i].y = word;
   }
 }
 
@@ -192,7 +260,7 @@ __global__ void k_tile_stats(dss2_graph_t g, int* stats) {
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct WsLayout {
-  size_t rowptr, col, eid, dis, w, ell_w, ell_ci, eptr, cursor, stats, cub, total, cub_bytes;
+  size_t rowptr, col, eid, dis, w, ell_w, ell_ci, hop_key, eptr, cursor, stats, cub, total, cub_bytes;
 };
 WsLayout ws_layout(int64_t Nt, int64_t Et, int32_t B) {
   WsLayout L;
@@ -205,6 +273,7 @@ WsLayout ws_layout(int64_t Nt, int64_t Et, int32_t B) {
   L.w = take((size_t)(2 * Et + 1) * 4);
   L.ell_w = take((size_t)(Nt + 1) * 16);
   L.ell_ci = take((size_t)(Nt + 1) * 8);
+  L.hop_key = take((size_t)(Nt + 1));
   L.eptr = take((size_t)(B + 1) * 8);
   L.cursor = take((size_t)(Nt + 1) * 4);
   L.stats = take(ST_COUNT * 4);
@@ -224,12 +293,13 @@ extern "C" size_t dss2_generic_scratch_bytes(int64_t Nt) { return ((size_t)4 * N
 extern "C" size_t dss2_graph_workspace_bytes(int64_t Nt, int64_t Et, int32_t B) { return ws_layout(Nt, Et, B).total; }
 
 extern "C" int dss2_graph_build(dss2_graph_t* g, const int64_t* edge_index, int64_t Et, int64_t Nt, const int64_t* ptr,
-                                int32_t B, int undirect, int tile_cap, void* ws, size_t ws_bytes, void* stream_) {
+                                int32_t B, int undirect, int tile_cap, int hop_keys, void* ws, size_t ws_bytes, void* stream_) {
   cudaStream_t stream = (cudaStream_t)stream_;
   DSS2_CHECK_ARG(g && ws && ptr && (edge_index || Et == 0), "dss2_graph_build: null argument");
   DSS2_CHECK_ARG(Nt >= 0 && Et >= 0 && B >= 1, "dss2_graph_build: bad sizes Nt=%lld Et=%lld B=%d", (long long)Nt, (long long)Et, B);
   DSS2_CHECK_ARG(Nt < (1LL << 31) - 2 && 2 * Et < (1LL << 31) - 2, "dss2_graph_build: batch too large for the int32 CSR");
   DSS2_CHECK_ARG(tile_cap >= 1 && tile_cap <= DSS2_TILE_CAP, "dss2_graph_build: tile_cap %d outside 1..%d", tile_cap, DSS2_TILE_CAP);
+  DSS2_CHECK_ARG(hop_keys == DSS2_HOP_KEYS_IDENTITY || hop_keys == DSS2_HOP_KEYS_COLOR, "dss2_graph_build: hop_keys %d is not a policy", hop_keys);
   WsLayout L = ws_layout(Nt, Et, B);
   DSS2_CHECK_ARG(ws_bytes >= L.total, "dss2_graph_build: workspace %zu < %zu bytes", ws_bytes, L.total);
   char* base = (char*)ws;
@@ -246,6 +316,8 @@ extern "C" int dss2_graph_build(dss2_graph_t* g, const int64_t* edge_index, int6
   g->w = (float*)(base + L.w);
   g->ell_w = (float*)(base + L.ell_w);
   g->ell_ci = (uint32_t*)(base + L.ell_ci);
+  g->hop_key = (uint8_t*)(base + L.hop_key);
+  g->hop_keys = hop_keys;
   g->eptr = (int64_t*)(base + L.eptr);
   int* cursor = (int*)(base + L.cursor);
   int* stats = (int*)(base + L.stats);
@@ -314,6 +386,19 @@ extern "C" int dss2_graph_build(dss2_graph_t* g, const int64_t* edge_index, int6
   g->max_tile_edges = h_stats[ST_MAX_TILE_EDGES];
   k_build_ell<<<g->num_tiles, 128, 0, stream>>>(*g);
   DSS2_LAUNCH_CHECK();
+  k_hop_keys<<<(g->num_tiles + 63) / 64, 64, 0, stream>>>(*g, hop_keys);
+  DSS2_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int dss2_hop_keys_host(const uint32_t* ell_ci, const int64_t* tile_ptr, int32_t num_tiles, int hop_keys, uint8_t* keys) {
+  DSS2_CHECK_ARG(ell_ci && tile_ptr && keys && num_tiles >= 0, "dss2_hop_keys_host: bad argument");
+  DSS2_CHECK_ARG(hop_keys == DSS2_HOP_KEYS_IDENTITY || hop_keys == DSS2_HOP_KEYS_COLOR, "dss2_hop_keys_host: hop_keys %d is not a policy", hop_keys);
+  for (int t = 0; t < num_tiles; ++t) {
+    const int64_t n0 = tile_ptr[t], nT = tile_ptr[t + 1] - n0;
+    DSS2_CHECK_ARG(nT >= 0 && nT <= DSS2_TILE_CAP, "dss2_hop_keys_host: tile %d has %lld rows", t, (long long)nT);
+    hop_keys_tile(reinterpret_cast<const uint2*>(ell_ci) + n0, (int)nT, (int)n0, hop_keys, keys + n0);
+  }
   return 0;
 }
 

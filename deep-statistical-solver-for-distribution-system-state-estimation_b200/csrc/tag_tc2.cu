@@ -171,10 +171,7 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS, Tc2Shape<RW>::CTAS_PER_
     // software pipeline over this CTA's tiles: node range two tiles ahead, rows + topology one tile ahead (all in registers)
     float xr[HF];
     uint32_t xr_bits = 0;
-    RowTopo tp_next;
-    tp_next.deg = 0;
-    tp_next.cols = 0;
-    tp_next.w = make_float4(0.f, 0.f, 0.f, 0.f);
+    RowTopo tp_next = row_topo(make_float4(0.f, 0.f, 0.f, 0.f), make_uint2(0u, 0u));
     auto load_row = [&](const TileNodes& tn) {   // this thread's half row of the tile, zero padded; BGX: masked grad_y
 #pragma unroll
       for (int i = 0; i < HF; ++i) xr[i] = 0.0f;
@@ -278,7 +275,7 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS, Tc2Shape<RW>::CTAS_PER_
             h[4 * q + 2] = v.z;
             h[4 * q + 3] = v.w;
           }
-        } else if (!DENSE && live) hop_thread(h, g, tp, lv_p(pb), n, n0, half);
+        } else if (!DENSE && live) hop_thread<false>(h, g, tp, lv_p(pb), n, n0, half);
         else {
 #pragma unroll
           for (int i = 0; i < HF; ++i) h[i] = 0.0f;
@@ -416,8 +413,9 @@ struct GwArgs {
   const float* gy;         // grad wrt layer output [Nt,cout]
   const uint32_t* bits;    // sign words or NULL
   const float* lvl;        // [K][Nt,32] = A g, A^2 g from the backward-to-input kernel
-  const uint32_t* lvl_fmt; // device word behind the levels: 0 = plain rows, 1 = rows as k_tag_tc3 spills them (16-byte chunk c of row n
-                           // stored at chunk c ^ (n & 7): byte image of its shared-memory tiles); NULL = plain
+  const uint32_t* lvl_fmt; // device words behind the levels: [0] = 0: plain rows; 1: rows as k_tag_tc3 spills them (byte image of its
+                           // shared-memory tiles: 16-byte chunk c of row n stored at chunk c ^ key[n]), with the key array (uint8 [Nt],
+                           // the graph's hop_key) as a pointer in words [2, 4).  NULL = plain
   int cout;
   float scale;
   float* partials;         // row = blockIdx.x
@@ -425,8 +423,13 @@ struct GwArgs {
   int64_t bias_offset;
 };
 
+// the key array of a spill in format 1, NULL for plain rows
+__device__ __forceinline__ const uint8_t* lvl_keys(const GwArgs& a) {
+  return a.lvl_fmt && a.lvl_fmt[0] == 1u ? *reinterpret_cast<const uint8_t* const*>(a.lvl_fmt + 2) : nullptr;
+}
+
 constexpr int GW_STAGES = 3;
-constexpr uint32_t GW_STAGE_BYTES = 4 * GW_TILE + 256;   // x, grad_y, A g, A^2 g rows + sign words of one 64-row chunk
+constexpr uint32_t GW_STAGE_BYTES = 4 * GW_TILE + 320;   // x, grad_y, A g, A^2 g rows + sign words + level swizzle keys of one 64-row chunk
 constexpr int GW_CONV = 512;                             // converter threads (16 warps): thread = (16-byte column chunk, row of the chunk)
 constexpr int GW_THREADS = GW_CONV + 64;                 // + 1 MMA-issuer warp + 1 bulk-copy producer warp
 // one operand buffer: A.hi[K+1 blocks] A.lo[K+1 blocks] B.hi B.lo.  The M = 128 descriptors span 4 blocks: the blocks past the K+1
@@ -487,7 +490,7 @@ __global__ void __launch_bounds__(GW_THREADS, 1) k_tag_gw(GwArgs a) {
 
   const int64_t num_chunks = (a.num_nodes + GW_ROWS - 1) / GW_ROWS;
   const int64_t full_chunks = a.num_nodes / GW_ROWS;       // only whole chunks go through the bulk-copy engine
-  const bool lvl_swz = a.lvl_fmt && *a.lvl_fmt == 1u;      // chunk rows start at multiples of 64, so (global row & 7) == (chunk row & 7)
+  const uint8_t* lvl_key = lvl_keys(a);
   float gb[4] = {0.f, 0.f, 0.f, 0.f};
   int it = 0;                                              // chunks this CTA has processed (same count in every role)
   // The tensor core adds into its fp32 accumulator with truncation, and a CTA adds ~500 MMAs into the same words: measured on the
@@ -504,7 +507,7 @@ __global__ void __launch_bounds__(GW_THREADS, 1) k_tag_gw(GwArgs a) {
   if (producer) {
     if (tc::elect_one()) {
       const uint32_t gy_bytes = (uint32_t)(GW_ROWS * cout * 4);
-      const uint32_t tx = GW_TILE * (K >= 2 ? 3 : 2) + gy_bytes + (a.bits ? 256u : 0u);
+      const uint32_t tx = GW_TILE * (K >= 2 ? 3 : 2) + gy_bytes + (a.bits ? 256u : 0u) + (lvl_key ? 64u : 0u);
       auto issue = [&](int64_t ch, int s) {
         if (ch >= full_chunks) return;
         char* st = stage0 + (size_t)s * GW_STAGE_BYTES;
@@ -515,6 +518,7 @@ __global__ void __launch_bounds__(GW_THREADS, 1) k_tag_gw(GwArgs a) {
         bulk_g2s(st + 2 * GW_TILE, a.lvl + n * 32, GW_TILE, &full[s]);
         if (K >= 2) bulk_g2s(st + 3 * GW_TILE, a.lvl + (a.num_nodes + n) * 32, GW_TILE, &full[s]);
         if (a.bits) bulk_g2s(st + 4 * GW_TILE, a.bits + n, 256, &full[s]);
+        if (lvl_key) bulk_g2s(st + 4 * GW_TILE + 256, lvl_key + n, 64, &full[s]);
       };
       for (int i = 0; i < GW_STAGES; ++i) issue(blockIdx.x + (int64_t)i * gridDim.x, i);
       for (int64_t ch = blockIdx.x; ch < num_chunks; ch += gridDim.x, ++it) {
@@ -578,7 +582,8 @@ __global__ void __launch_bounds__(GW_THREADS, 1) k_tag_gw(GwArgs a) {
       float4 vx, vg, v1, v2;
       vx = vg = v1 = v2 = make_float4(0.f, 0.f, 0.f, 0.f);
       uint32_t word = 0xffffffffu;
-      const uint32_t cl = cq ^ (lvl_swz ? (r & 7u) : 0u);   // chunk position of columns [4 cq, 4 cq + 4) in a spilled level row
+      uint32_t cl = cq;   // chunk position of columns [4 cq, 4 cq + 4) in a spilled level row
+      if (lvl_key) cl ^= staged ? (uint32_t)reinterpret_cast<const uint8_t*>(st + 4 * GW_TILE + 256)[r] : n < a.num_nodes ? (uint32_t)lvl_key[n] : 0u;
       if (staged) {
         vx = *reinterpret_cast<const float4*>(st + r * 128 + cq * 16);
         v1 = *reinterpret_cast<const float4*>(st + 2 * GW_TILE + r * 128 + cl * 16);
@@ -688,7 +693,7 @@ __global__ void __launch_bounds__(GW_THREADS, 1) k_tag_gw(GwArgs a) {
 // -------------------------------------------------------------------------------------------------
 constexpr int GWF_STAGES = 4;
 constexpr int GWF_THREADS = 256;
-#define GWF_STAGE_BYTES(K) ((uint32_t)((K) + 2) * GW_TILE + 256u)   // x, grad_y, K hop levels, sign words
+#define GWF_STAGE_BYTES(K) ((uint32_t)((K) + 2) * GW_TILE + 320u)   // x, grad_y, K hop levels, sign words, level swizzle keys
 template <int K>
 size_t gwf_smem() { return 1024 + GWF_STAGES * GWF_STAGE_BYTES(K) + 2 * GW_TILE + 32 * 33 * 4 + 64; }
 
@@ -711,7 +716,8 @@ __global__ void __launch_bounds__(GWF_THREADS, 1) k_tag_gw_ffma(GwArgs a) {
   const int64_t num_chunks = (a.num_nodes + GW_ROWS - 1) / GW_ROWS;
   const int64_t full_chunks = a.num_nodes / GW_ROWS;
   const uint32_t gy_bytes = (uint32_t)(GW_ROWS * cout * 4);
-  const uint32_t tx = GW_TILE * (K + 1) + gy_bytes + (a.bits ? 256u : 0u);
+  const uint8_t* lvl_key = lvl_keys(a);
+  const uint32_t tx = GW_TILE * (K + 1) + gy_bytes + (a.bits ? 256u : 0u) + (lvl_key ? 64u : 0u);
   auto issue = [&](int64_t ch, int s) {
     if (ch >= full_chunks) return;
     char* st = stage0 + (size_t)s * STAGE;
@@ -722,13 +728,13 @@ __global__ void __launch_bounds__(GWF_THREADS, 1) k_tag_gw_ffma(GwArgs a) {
 #pragma unroll
     for (int k = 0; k < K; ++k) bulk_g2s(st + (2 + k) * GW_TILE, a.lvl + ((int64_t)k * a.num_nodes + n) * 32, GW_TILE, &full[s]);
     if (a.bits) bulk_g2s(st + (K + 2) * GW_TILE, a.bits + n, 256, &full[s]);
+    if (lvl_key) bulk_g2s(st + (K + 2) * GW_TILE + 256, lvl_key + n, 64, &full[s]);
   };
   if (tid == 0)
     for (int i = 0; i < GWF_STAGES - 1; ++i) issue(blockIdx.x + (int64_t)i * gridDim.x, i);
 
   const uint32_t cq = tid & 7, rs = tid >> 3;          // pre-pass mapping: 16-byte column chunk, row (and row + 32)
   const int i_feat = tid & 31, c0 = (tid >> 5) * 4;    // main mapping
-  const bool lvl_swz = a.lvl_fmt && *a.lvl_fmt == 1u;
   float gb[4] = {0.f, 0.f, 0.f, 0.f};
   float acc[K + 1][4];
 #pragma unroll
@@ -754,6 +760,7 @@ __global__ void __launch_bounds__(GWF_THREADS, 1) k_tag_gw_ffma(GwArgs a) {
           reinterpret_cast<float*>(st + (2 + k) * GW_TILE)[idx] = inb ? a.lvl[((int64_t)k * a.num_nodes + n0 + r) * 32 + j] : 0.0f;   // byte image: keeps the level format
         if (j < cout) reinterpret_cast<float*>(st + GW_TILE)[r * cout + j] = inb ? a.gy[(n0 + r) * cout + j] : 0.0f;
         if (a.bits && j == 0) reinterpret_cast<uint32_t*>(st + (K + 2) * GW_TILE)[r] = inb ? a.bits[n0 + r] : 0u;
+        if (lvl_key && j == 0) reinterpret_cast<uint8_t*>(st + (K + 2) * GW_TILE + 256)[r] = inb ? lvl_key[n0 + r] : 0u;
       }
       __syncthreads();
     }
@@ -788,9 +795,11 @@ __global__ void __launch_bounds__(GWF_THREADS, 1) k_tag_gw_ffma(GwArgs a) {
     __syncthreads();   // g0 complete; every thread has left the main loop of the previous chunk -> its slot may be refilled
     if (tid == 0) issue(ch + (int64_t)(GWF_STAGES - 1) * gridDim.x, (it + GWF_STAGES - 1) % GWF_STAGES);
     const float* xs = reinterpret_cast<const float*>(st) + i_feat;
+    const uint8_t* ks = reinterpret_cast<const uint8_t*>(st + (K + 2) * GW_TILE + 256);
 #pragma unroll 4
     for (int r = 0; r < GW_ROWS; ++r) {
       const float xv = xs[r * 32];
+      const uint32_t cl = (uint32_t)(c0 >> 2) ^ (lvl_key ? (uint32_t)ks[r] : 0u);
       const float4 l0 = *reinterpret_cast<const float4*>(g0 + r * 32 + c0);
       acc[0][0] = fmaf(l0.x, xv, acc[0][0]);
       acc[0][1] = fmaf(l0.y, xv, acc[0][1]);
@@ -798,7 +807,7 @@ __global__ void __launch_bounds__(GWF_THREADS, 1) k_tag_gw_ffma(GwArgs a) {
       acc[0][3] = fmaf(l0.w, xv, acc[0][3]);
 #pragma unroll
       for (int k = 1; k <= K; ++k) {
-        const float4 lk = *reinterpret_cast<const float4*>(st + (1 + k) * GW_TILE + r * 128 + (((uint32_t)(c0 >> 2) ^ (lvl_swz ? (uint32_t)(r & 7) : 0u)) << 4));
+        const float4 lk = *reinterpret_cast<const float4*>(st + (1 + k) * GW_TILE + r * 128 + (cl << 4));
         acc[k][0] = fmaf(lk.x, xv, acc[k][0]);
         acc[k][1] = fmaf(lk.y, xv, acc[k][1]);
         acc[k][2] = fmaf(lk.z, xv, acc[k][2]);

@@ -10,9 +10,9 @@
 //     the sign words with 1-D bulk copies; the tile's node range travels through shared memory with them, so a worker issues no
 //     global load at all;
 //   * the backward's hop levels leave as ONE cp.async.bulk store per level straight from the plain level tile the next hop
-//     gathers from.  That tile is software-swizzled by the GLOBAL row (16-byte chunk c of row n sits at chunk c ^ (n & 7)), so its
-//     byte image in global memory can be un-swizzled by the weight-gradient kernel without knowing the tiling (format word 1
-//     behind the levels, see GwArgs::lvl_fmt);
+//     gathers from.  That tile is software-swizzled by the graph's per-row keys (16-byte chunk c of row n sits at chunk
+//     c ^ hop_key[n], see DSS2_HOP_KEYS_COLOR), so its byte image in global memory can be un-swizzled by the weight-gradient kernel
+//     without knowing the tiling (format word 1 and the key array behind the levels, see GwArgs::lvl_fmt);
 //   * the A operand lives in tensor memory as in k_tag_tc2<TA> (tcgen05.st by the thread that owns the row), so shared memory is
 //     read by generic-proxy gathers only and the sole proxy fence left is the one in front of the spill (cheap now: a worker has
 //     no global access in flight when it executes it).
@@ -150,7 +150,11 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
       mbar_init(&sp_done[i], 1);
     }
     fence_mbar_init();
-    if (spill && blockIdx.x == 0) *reinterpret_cast<uint32_t*>(a.lvl_out + (size_t)K * g.num_nodes * 32) = 1u;   // spill format: swizzled rows
+    if (spill && blockIdx.x == 0) {   // spill format: rows swizzled by the keys in g.hop_key
+      uint32_t* fmt = reinterpret_cast<uint32_t*>(a.lvl_out + (size_t)K * g.num_nodes * 32);
+      fmt[0] = 1u;
+      *reinterpret_cast<const uint8_t**>(fmt + 2) = g.hop_key;
+    }
   }
   if (warp == 0) tc::tmem_alloc(tslot, TMEM_COLS);
   // land tile `tn` in stage s; the node range goes with it (written before the arrive.expect_tx, which releases it)
@@ -296,7 +300,6 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
     // ===== worker warps: thread = (row, half) =====
     uint32_t par[2] = {0u, 0u}, ipar[2] = {0u, 0u}, spar[2] = {0u, 0u};
     const uint32_t tlane = (uint32_t)((warp & 3) * 32) << 16;
-    uint32_t phase = 0;   // n0 & 7 of the current tile: software swizzle key of the plain level tiles = global row & 7
     auto publish = [&](int b, bool meet, bool spilled) {
       if (spilled) fence_proxy_async();   // the bulk store reads this thread's STS through the async proxy
       tc::tmem_wait_st();
@@ -304,9 +307,9 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
       tc::mbar_arrive(&full[b]);
       if (meet) named_bar_sync(1, WORKERS);
     };
-    auto store_level = [&](const float (&v)[HF], int b, bool to_smem) {
+    auto store_level = [&](const float (&v)[HF], uint32_t key, int b, bool to_smem) {
       if (to_smem) {
-        const uint32_t code = row_code_ph(row, phase);
+        const uint32_t code = row_code_key(row, key);
         char* pt = Lv + (size_t)b * LV_TILE;
 #pragma unroll
         for (uint32_t q = 0; q < 4; ++q)
@@ -333,7 +336,6 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
       const int n0 = tinfo[2 * s], nT = tinfo[2 * s + 1] - n0;
       const bool live = (int)row < nT;
       const size_t n = (size_t)n0 + row;
-      phase = (uint32_t)n0 & 7u;
       // ---- this thread's half row and topology out of the stage (the tensor map swizzles by the stage row) ----
       float xr[HF];
       RowTopo tp;
@@ -366,10 +368,8 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
             xr[4 * q + 3] = v.w;
           }
         }
-        tp.w = *reinterpret_cast<const float4*>(st + Sm::ST_W + row * 16);
-        const uint2 ci = *reinterpret_cast<const uint2*>(st + Sm::ST_CI + ((uint32_t)(n0 & 1) + row) * 8);
-        tp.cols = ci.x;
-        tp.deg = ci.y;
+        tp = row_topo(*reinterpret_cast<const float4*>(st + Sm::ST_W + row * 16),
+                      *reinterpret_cast<const uint2*>(st + Sm::ST_CI + ((uint32_t)(n0 & 1) + row) * 8));
         uint32_t word = 0xffffu;
         if (has_bits) word = *reinterpret_cast<const uint32_t*>(st + Sm::ST_BITS + ((uint32_t)(n0 & 3) + row) * 4) >> (half * HF);
         if (!live) word = 0u;   // rows past the tile hold the next tile's data: the MMA input of dead rows is zero
@@ -385,7 +385,8 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
         mbar_wait(&sp_done[0], spar[0]);
         spar[0] ^= 1u;
       }
-      store_level(xr, 0, true);
+      const uint32_t skey = tp.keys & 7u;   // this row's swizzle key in the plain level tiles
+      store_level(xr, skey, 0, true);
       STAMP(1);   // stage read + store L0
       publish(0, true, false);
       STAMP(2);
@@ -394,7 +395,7 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
       for (int k = 1; k <= K; ++k) {
         const int b = k & 1, pb = (k - 1) & 1;
         float h[HF];
-        if (live) hop_thread(h, g, tp, Lv + (size_t)pb * LV_TILE, n, n0, half, phase);
+        if (live) hop_thread<true>(h, g, tp, Lv + (size_t)pb * LV_TILE, n, n0, half);
         else {
 #pragma unroll
           for (int i = 0; i < HF; ++i) h[i] = 0.0f;
@@ -409,7 +410,7 @@ __global__ void __launch_bounds__(Tc2Shape<RW>::THREADS + 32, RW == 8 ? 1 : 2) k
           spar[1] ^= 1u;
         }
         STAMP(4 + 4 * (k - 1));
-        store_level(h, b, k < K || spill);
+        store_level(h, skey, b, k < K || spill);
         STAMP(5 + 4 * (k - 1));
         publish(b, k < K, spill);
         STAMP(6 + 4 * (k - 1));

@@ -61,12 +61,11 @@ __device__ __forceinline__ void store_half_sw128(const float (&v)[HF], char* pt,
     tc::plain_store4(make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]), pt, lt, code ^ ((half * 4 + q) << 4));
 }
 
-// h += w * plain[src row][16*half ...]: one neighbour, exact fp32 values from the plain tile
-// `phase`: the tile's swizzle key offset - 0 for hardware-swizzled tiles (key = tile-local row), n0 & 7 for the software-swizzled
-// plain tiles of k_tag_tc3 (key = GLOBAL row, so that a tile copied to global memory byte for byte can be un-swizzled by anyone)
-__device__ __forceinline__ uint32_t row_code_ph(uint32_t row, uint32_t phase) { return (row << 7) | (((row + phase) & 7u) << 4); }
-__device__ __forceinline__ void gather_half(float (&h)[HF], const char* pt, uint32_t src, float w, uint32_t half, uint32_t phase = 0) {
-  const uint32_t code = row_code_ph(src, phase);
+// h += w * plain[src row][16*half ...]: one neighbour, exact fp32 values from the plain tile, whose 16-byte chunk c of row `src` sits at
+// chunk c ^ key (key = src & 7 in the hardware-swizzled tiles of k_tag_tc2, the row's swizzle key in the plain tiles of k_tag_tc3)
+__device__ __forceinline__ uint32_t row_code_key(uint32_t row, uint32_t key) { return (row << 7) | (key << 4); }
+__device__ __forceinline__ void gather_half(float (&h)[HF], const char* pt, uint32_t src, uint32_t key, float w, uint32_t half) {
+  const uint32_t code = row_code_key(src, key);
 #pragma unroll
   for (uint32_t q = 0; q < 4; ++q) {
     const float4 a = *reinterpret_cast<const float4*>(pt + (code ^ ((half * 4 + q) << 4)));
@@ -80,29 +79,40 @@ __device__ __forceinline__ void gather_half(float (&h)[HF], const char* pt, uint
 struct RowTopo {
   float4 w;        // weights of the first 4 entries
   uint32_t cols;   // 4 x 8-bit tile-local sources
-  uint32_t deg;
+  uint32_t deg;    // degree (saturated at DSS2_ELL_DEG_MASK: hub rows take their extent from rowptr)
+  uint32_t keys;   // swizzle keys: bits 0..2 the row's own, 3 + 3d..5 + 3d those of ELL source d
 };
-__device__ __forceinline__ RowTopo load_row_topo(const dss2_graph_t& g, size_t n) {
+__device__ __forceinline__ RowTopo row_topo(float4 w, uint2 ci) {
   RowTopo t;
-  t.w = reinterpret_cast<const float4*>(g.ell_w)[n];
-  const uint2 ci = reinterpret_cast<const uint2*>(g.ell_ci)[n];
+  t.w = w;
   t.cols = ci.x;
-  t.deg = ci.y;
+  t.deg = ci.y & DSS2_ELL_DEG_MASK;
+  t.keys = ci.y >> DSS2_ELL_KEY_SHIFT;
   return t;
 }
+__device__ __forceinline__ RowTopo load_row_topo(const dss2_graph_t& g, size_t n) {
+  return row_topo(reinterpret_cast<const float4*>(g.ell_w)[n], reinterpret_cast<const uint2*>(g.ell_ci)[n]);
+}
 
-// one hop for this thread's half row: entries in CSR order = PyG scatter order
+// one hop for this thread's half row: entries in CSR order = PyG scatter order.  BUS_KEYS: the plain tile is swizzled by the graph's
+// per-row keys (k_tag_tc3), else by the tile row (k_tag_tc2's hardware swizzle)
+template <bool BUS_KEYS>
 __device__ __forceinline__ void hop_thread(float (&h)[HF], const dss2_graph_t& g, const RowTopo& tp, const char* pt, size_t n, int n0,
-                                           uint32_t half, uint32_t phase = 0) {
+                                           uint32_t half) {
 #pragma unroll
   for (int i = 0; i < HF; ++i) h[i] = 0.0f;
   const float wv[4] = {tp.w.x, tp.w.y, tp.w.z, tp.w.w};
 #pragma unroll
-  for (uint32_t d = 0; d < 4; ++d)
-    if (d < tp.deg) gather_half(h, pt, (tp.cols >> (8 * d)) & 0xffu, wv[d], half, phase);
+  for (uint32_t d = 0; d < 4; ++d) {
+    const uint32_t src = (tp.cols >> (8 * d)) & 0xffu;
+    if (d < tp.deg) gather_half(h, pt, src, BUS_KEYS ? (tp.keys >> (3 + 3 * d)) & 7u : src & 7u, wv[d], half);
+  }
   if (tp.deg > 4) {   // rare: hub nodes
-    const int beg = g.rowptr[n];
-    for (int z = beg + 4; z < beg + (int)tp.deg; ++z) gather_half(h, pt, (uint32_t)(g.col[z] - n0), g.w[z], half, phase);
+    const int beg = g.rowptr[n], end = g.rowptr[n + 1];
+    for (int z = beg + 4; z < end; ++z) {
+      const int c = g.col[z];
+      gather_half(h, pt, (uint32_t)(c - n0), BUS_KEYS ? (uint32_t)g.hop_key[c] : (uint32_t)(c - n0) & 7u, g.w[z], half);
+    }
   }
 }
 

@@ -14,6 +14,18 @@ LIB_PATH = os.path.join(os.path.dirname(_HERE), "csrc", "libdss2_b200.so")
 
 HID = 32
 TILE_CAP = 256
+# swizzle-key policies of dss2_graph_build (DSS2_HOP_KEYS_* in the header)
+HOP_KEYS = {"identity": 0, "color": 1}
+ELL_DEG_MASK = 0x1FFFF
+ELL_KEY_SHIFT = 17
+
+
+def hop_keys_default():
+    """Policy for graphs built without an explicit one: $DSS2_HOP_KEYS (identity | color), read at every build; color when unset."""
+    name = os.environ.get("DSS2_HOP_KEYS", "color")
+    if name not in HOP_KEYS:
+        raise ValueError(f"DSS2_HOP_KEYS={name!r}: expected one of {sorted(HOP_KEYS)}")
+    return name
 
 
 class GraphStruct(Structure):
@@ -21,10 +33,10 @@ class GraphStruct(Structure):
     _fields_ = [
         ("num_nodes", c_int64), ("num_edges", c_int64), ("nnz", c_int64),
         ("num_graphs", c_int32), ("undirected", c_int32), ("graphs_per_tile", c_int32), ("num_tiles", c_int32),
-        ("max_tile_nodes", c_int32), ("max_tile_nnz", c_int32), ("max_tile_edges", c_int32), ("reserved", c_int32),
+        ("max_tile_nodes", c_int32), ("max_tile_nnz", c_int32), ("max_tile_edges", c_int32), ("hop_keys", c_int32),
         ("edge_index", c_void_p), ("ptr", c_void_p), ("eptr", c_void_p), ("rowptr", c_void_p), ("col", c_void_p),
         ("eid", c_void_p), ("dis", c_void_p), ("w", c_void_p), ("ell_w", c_void_p), ("ell_ci", c_void_p),
-        ("scratch", c_void_p), ("scratch_bytes", c_size_t),
+        ("scratch", c_void_p), ("scratch_bytes", c_size_t), ("hop_key", c_void_p),
     ]
 
 
@@ -54,7 +66,8 @@ _SIGNATURES = {
     "dss2_launch_count": (c_int64, []),
     "dss2_graph_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int32]),
     "dss2_generic_scratch_bytes": (c_size_t, [c_int64]),
-    "dss2_graph_build": (c_int, [_G, _P, c_int64, c_int64, _P, c_int32, c_int, c_int, _P, c_size_t, _P]),
+    "dss2_graph_build": (c_int, [_G, _P, c_int64, c_int64, _P, c_int32, c_int, c_int, c_int, _P, c_size_t, _P]),
+    "dss2_hop_keys_host": (c_int, [_P, _P, c_int32, c_int, _P]),
     "dss2_pack_batch": (c_int, [_P, _P, _P, _P, c_int64, _P, _P, _P, c_int32, _P, _P, c_int64, _P, _P, _P, _P, _P, _P, _P]),
     "dss2_col_minmax": (c_int, [_P, c_int64, c_int, c_int64, _P, _P]),
     "dss2_edgeagg_fwd": (c_int, [_G, _P, c_int64, c_int, _P, c_int64, c_int, _P, _P, _P, _P, _P, _P]),

@@ -121,7 +121,7 @@ def pack_batch(store, ids, graph_cache=None):
         # structure: identical for every batch drawn from a uniform-topology store with the same graph count
         key = None
         if graph_cache is not None and _uniform(store):
-            key = (b, store.max_nodes, store.max_edges, _tile_cap())
+            key = (b, store.max_nodes, store.max_edges, _tile_cap(), _lib.hop_keys_default())
         g = graph_cache.get(key) if key is not None else None
         if g is None:
             if key is not None:

@@ -8,6 +8,7 @@ the edge_index tensor); foreign tensors get one built on first use.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -16,8 +17,13 @@ from . import _lib
 class BatchGraph:
     """Owns the device workspace behind a `dss2_graph_t`."""
 
-    def __init__(self, edge_index, num_nodes, ptr=None, undirect=-1, tile_cap=_lib.TILE_CAP):
+    def __init__(self, edge_index, num_nodes, ptr=None, undirect=-1, tile_cap=_lib.TILE_CAP, hop_keys=None):
+        """hop_keys: swizzle-key policy of the layer kernels' shared-memory tiles ("identity" or "color", see
+        DSS2_HOP_KEYS_COLOR in dss2_b200.h); None = `_lib.hop_keys_default()`.  Results do not depend on it."""
         lib = _lib.load()
+        self.hop_keys = _lib.hop_keys_default() if hop_keys is None else hop_keys
+        if self.hop_keys not in _lib.HOP_KEYS:
+            raise ValueError(f"hop_keys={self.hop_keys!r}: expected one of {sorted(_lib.HOP_KEYS)}")
         if edge_index.device.type != "cuda":
             raise _lib.Dss2Error("BatchGraph needs CUDA tensors")
         if edge_index.dtype != torch.long or edge_index.dim() != 2 or edge_index.size(0) != 2:
@@ -35,7 +41,8 @@ class BatchGraph:
         self.c = _lib.GraphStruct()
         with torch.cuda.device(edge_index.device):
             rc = lib.dss2_graph_build(ctypes.byref(self.c), _lib.ptr(self.edge_index), self.num_edges, self.num_nodes,
-                                      _lib.ptr(self.ptr), self.num_graphs, undirect, tile_cap, _lib.ptr(self.ws), nbytes,
+                                      _lib.ptr(self.ptr), self.num_graphs, undirect, tile_cap, _lib.HOP_KEYS[self.hop_keys],
+                                      _lib.ptr(self.ws), nbytes,
                                       _lib.stream())
         _lib.check(rc, "dss2_graph_build")
         self._wls_ws = None
@@ -73,6 +80,8 @@ class BatchGraph:
             "rowptr": view(c.rowptr, c.num_nodes + 1, torch.int32), "col": view(c.col, c.nnz, torch.int32),
             "eid": view(c.eid, c.nnz, torch.int32), "dis": view(c.dis, c.num_nodes, torch.float32),
             "eptr": view(c.eptr, c.num_graphs + 1, torch.int64), "w": view(c.w, c.nnz, torch.float32),
+            "ell_ci": view(c.ell_ci, 2 * c.num_nodes if c.num_tiles else 0, torch.int32),
+            "hop_key": view(c.hop_key, c.num_nodes if c.num_tiles else 0, torch.uint8),
         }
 
 
@@ -96,7 +105,8 @@ def discover_segments(edge_index, num_nodes):
 def graph_for(edge_index, num_nodes):
     """The cached BatchGraph attached to `edge_index`, building (and attaching) it if needed."""
     g = getattr(edge_index, "_dss2_graph", None)
-    if g is not None and g.num_nodes == num_nodes and g.edge_index.data_ptr() == edge_index.data_ptr():
+    if (g is not None and g.num_nodes == num_nodes and g.edge_index.data_ptr() == edge_index.data_ptr()
+            and g.hop_keys == _lib.hop_keys_default()):
         return g
     g = BatchGraph(edge_index, num_nodes)
     try:
@@ -104,3 +114,73 @@ def graph_for(edge_index, num_nodes):
     except AttributeError:
         pass
     return g
+
+
+# ---- host model of the tiling, the ELL view and the swizzle keys of dss2_graph_build (tests, tools/hop_conflicts.py) ----
+
+def host_ell(edge_index, ptr, tile_cap=_lib.TILE_CAP, undirect=True):
+    """(ell_ci uint32 [Nt, 2], tile_ptr int64 [num_tiles + 1]) as dss2_graph_build makes them before packing the keys: column 0 =
+    4 x 8-bit tile-local sources of a row's first 4 entries in PyG scatter order (padding = the row itself), column 1 = degree.
+    None when a graph exceeds `tile_cap`."""
+    ei = np.asarray(edge_index, dtype=np.int64)
+    ptr = np.asarray(ptr, dtype=np.int64)
+    nt, b = int(ptr[-1]), len(ptr) - 1
+    seg = int(np.diff(ptr).max())
+    if seg == 0 or seg > tile_cap:
+        return None
+    src, dst = (np.concatenate([ei[0], ei[1]]), np.concatenate([ei[1], ei[0]])) if undirect else (ei[0], ei[1])
+    order = np.lexsort((np.arange(dst.size), dst))    # by destination, then by doubled edge id
+    src, dst = src[order], dst[order]
+    deg = np.bincount(dst, minlength=nt)
+    rowptr = np.concatenate([[0], np.cumsum(deg)])
+    per = tile_cap // seg
+    tile_ptr = ptr[np.r_[np.arange(0, b, per), b]]
+    n0 = np.repeat(tile_ptr[:-1], np.diff(tile_ptr))
+    rows = np.arange(nt)
+    ci = np.zeros((nt, 2), dtype=np.uint32)
+    for d in range(4):
+        has = deg > d
+        col = rows.copy()
+        col[has] = src[rowptr[:-1][has] + d]
+        ci[:, 0] |= (((col - n0) & 0xff) << (8 * d)).astype(np.uint32)
+    ci[:, 1] = np.minimum(deg, _lib.ELL_DEG_MASK)
+    return ci, tile_ptr
+
+
+def host_hop_keys(ell_ci, tile_ptr, policy):
+    """The keys (uint8 [Nt]) dss2_graph_build assigns under `policy` ("identity" or "color"), computed by the library on the host."""
+    ci = np.ascontiguousarray(ell_ci, dtype=np.uint32)
+    tp = np.ascontiguousarray(tile_ptr, dtype=np.int64)
+    keys = np.zeros(ci.shape[0], dtype=np.uint8)
+    lib = _lib.load(require_cuda=False)
+    _lib.check(lib.dss2_hop_keys_host(ci.ctypes.data, tp.ctypes.data, len(tp) - 1, _lib.HOP_KEYS[policy], keys.ctypes.data),
+               "dss2_hop_keys_host")
+    return keys
+
+
+def hop_wavefronts(ell_ci, tile_ptr, keys):
+    """Shared-memory wavefronts of the layer kernels' 128-bit accesses to the plain level tiles, against the conflict-free count:
+    {"gather": (wavefronts, ideal), "store": (wavefronts, ideal)}.  One access phase = 8 consecutive rows of a tile; rows with
+    different addresses and equal keys share banks, so a phase takes as many wavefronts as the most frequent key among its
+    distinct rows (gathers: the rows' active slot-d sources, one count per slot; stores: the rows themselves)."""
+    ci = np.asarray(ell_ci, dtype=np.uint32)
+    tile_ptr = np.asarray(tile_ptr, dtype=np.int64)
+    keys = np.asarray(keys, dtype=np.int64)
+    n0 = np.repeat(tile_ptr[:-1], np.diff(tile_ptr))
+    rows = np.arange(ci.shape[0])
+    group = np.repeat(np.arange(len(tile_ptr) - 1), np.diff(tile_ptr)) * (_lib.TILE_CAP // 8) + (rows - n0) // 8
+
+    def waves(grp, member):
+        u = np.unique(np.stack([grp, member]), axis=1)               # distinct rows per phase
+        gk = np.unique(np.stack([u[0], keys[u[1]]]), axis=1, return_counts=True)
+        per = np.zeros(int(grp.max()) + 1, dtype=np.int64)
+        np.maximum.at(per, gk[0][0], gk[1])
+        return int(per.sum()), int(np.count_nonzero(per))
+
+    deg = np.minimum(ci[:, 1] & _lib.ELL_DEG_MASK, 4)
+    gg, gm = [], []
+    for d in range(4):
+        act = deg > d
+        gg.append(group[act] * 4 + d)
+        gm.append(n0[act] + ((ci[act, 0] >> (8 * d)) & 0xff))
+    return {"gather": waves(np.concatenate(gg), np.concatenate(gm)), "store": waves(group, rows)}

@@ -428,7 +428,7 @@ def resolve_graph(edge_index, num_nodes):
     """BatchGraph for `edge_index` (CPU or CUDA).  Cached on the tensor object, keyed by its version."""
     cached = getattr(edge_index, "_dss2_graph", None)
     if (cached is not None and cached.num_nodes == num_nodes and getattr(edge_index, "_dss2_graph_version", None) == edge_index._version
-            and cached.tile_cap <= tile_cap()):
+            and cached.tile_cap <= tile_cap() and cached.hop_keys == _lib.hop_keys_default()):
         return cached
     ei = edge_index if edge_index.device.type == "cuda" else edge_index.cuda(non_blocking=True)
     g = BatchGraph(ei.long(), num_nodes, ptr=getattr(edge_index, "_dss2_ptr", None), tile_cap=tile_cap())

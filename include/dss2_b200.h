@@ -53,7 +53,7 @@ typedef struct dss2_graph {
   int32_t max_tile_nodes;
   int32_t max_tile_nnz;
   int32_t max_tile_edges;   /* one-way edges */
-  int32_t reserved;
+  int32_t hop_keys;         /* swizzle-key policy the build used (DSS2_HOP_KEYS_*) */
   const int64_t* edge_index;/* [2,Et] caller's tensor */
   const int64_t* ptr;       /* [B+1] node offset of every graph (caller's or builder's) */
   int64_t* eptr;            /* [B+1] one-way edge offset of every graph */
@@ -63,10 +63,22 @@ typedef struct dss2_graph {
   float* dis;               /* [Nt] in-degree^-1/2 on the doubled graph, 0 where degree is 0 */
   float* w;                 /* [nnz] gcn_norm weight of the entry: dis[src] * dis[dst] */
   float* ell_w;             /* [Nt][4] weights of the first 4 entries of every row (0 = padding): thread-per-row kernels */
-  uint32_t* ell_ci;         /* [Nt][2] .x = 4 x 8-bit tile-local source rows of those entries, .y = row degree */
+  uint32_t* ell_ci;         /* [Nt][2] .x = 4 x 8-bit tile-local source rows of those entries, .y = row degree (saturated at
+                               DSS2_ELL_DEG_MASK) | swizzle keys of the row and of its 4 ELL sources (DSS2_ELL_KEY_SHIFT) */
   float* scratch;           /* caller-provided, only needed when num_tiles == 0 (a graph exceeds a tile): */
   size_t scratch_bytes;     /*   dss2_generic_scratch_bytes(Nt) bytes of device memory for the large-graph kernels */
+  uint8_t* hop_key;         /* [Nt] swizzle key (0..7) of every row of a tiled graph */
 } dss2_graph_t;
+
+/* Swizzle keys.  The TAG layer kernels keep each hop level of a tile in shared memory as 128-byte rows, with 16-byte chunk c of
+ * row n stored at chunk c ^ key[n].  Eight consecutive tile rows form one phase of a 128-bit shared-memory access, so rows whose
+ * keys differ never share banks.  IDENTITY: key = n & 7 (consecutive rows differ).  COLOR: keys chosen per tile at graph build so
+ * that the rows gathered together by one phase (the slot-d ELL sources of 8 consecutive rows) differ as well.  The keys move
+ * bytes only: every sum, and so every result, is the same under both policies. */
+#define DSS2_HOP_KEYS_IDENTITY 0
+#define DSS2_HOP_KEYS_COLOR 1
+#define DSS2_ELL_DEG_MASK 0x1ffffu   /* ell_ci[n].y bits 0..16: degree; 17..19: key of n; 20 + 3d..22 + 3d: key of ELL source d */
+#define DSS2_ELL_KEY_SHIFT 17
 
 /* Large graphs (a graph with more nodes than a tile, e.g. a 10k-bus feeder): num_tiles == 0 after the build and every layer /
  * loss entry point switches to its global-memory variant (hops as separate SpMM launches, row-streaming transforms, node-centric
@@ -79,10 +91,15 @@ size_t dss2_graph_workspace_bytes(int64_t num_nodes, int64_t num_edges, int32_t 
 /* Builds the structure into `g` (host struct).  `ws` must stay alive as long as `g` is used: all
  * arrays of `g` except edge_index/ptr point into it.  undirect: 1 append reversed edges, 0 do not,
  * -1 decide like MPN.is_directed (networks.py:236-238).  tile_cap: max nodes per tile (<= DSS2_TILE_CAP).
+ * hop_keys: DSS2_HOP_KEYS_IDENTITY or DSS2_HOP_KEYS_COLOR.
  * Synchronises `stream` (reads sizes back); not graph-capturable. */
 int dss2_graph_build(dss2_graph_t* g, const int64_t* edge_index, int64_t num_edges, int64_t num_nodes,
-                     const int64_t* ptr, int32_t num_graphs, int undirect, int tile_cap,
+                     const int64_t* ptr, int32_t num_graphs, int undirect, int tile_cap, int hop_keys,
                      void* ws, size_t ws_bytes, void* stream);
+
+/* The keys dss2_graph_build assigns, computed on the host (tests, tools/hop_conflicts.py).  All pointers are HOST pointers:
+ * ell_ci [Nt][2] = the ELL words with the plain degree in .y, tile_ptr [num_tiles+1] = first row of every tile; keys [Nt] out. */
+int dss2_hop_keys_host(const uint32_t* ell_ci, const int64_t* tile_ptr, int32_t num_tiles, int hop_keys, uint8_t* keys);
 
 /* ------------------------------------------------------------------------------------------------
  * (a) Batch packer.  Replaces PyG DataLoader -> Batch.from_data_list (dss2_run.py:18,68-69,134).
@@ -164,7 +181,8 @@ int dss2_tag_fwd(const dss2_graph_t* g, const float* x, const float* w, const fl
  * backward-to-input for cout == 32), else k_tag_tc2 with direct loads (DSS2_TC3=0 forces that).  Contract details of the TMA path:
  * act_bits buffers hold (num_nodes + 3) & ~3 words (the sign words of a tile are copied from a 16-byte aligned start);
  * the last 256 bytes of the backward workspace carry a format word written by _gx and read by _gw / dss2_tag_gw_ffma (0 = plain
- * level rows, 1 = rows whose 16-byte chunk c is stored at chunk c ^ (row & 7)): pass the SAME workspace to both. */
+ * level rows, 1 = rows whose 16-byte chunk c is stored at chunk c ^ g->hop_key[row], followed by that key array's address):
+ * pass the SAME workspace to both, while the graph is alive. */
 int dss2_tag_tc2_supported(const dss2_graph_t* g, int K);
 int dss2_tag_fwd_tc2(const dss2_graph_t* g, const float* x, const float* w, const float* bias, int cout, int K,
                      int act, float p_drop, int drop_mode, const uint64_t* rng_state, uint32_t layer_uid,
