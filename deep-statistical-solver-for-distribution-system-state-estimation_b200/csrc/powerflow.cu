@@ -11,6 +11,7 @@
 // converged = 0 for that scenario only.
 #include <math.h>
 
+#include "block_lu.cuh"
 #include "common.cuh"
 
 namespace {
@@ -29,25 +30,6 @@ struct PfArgs {
   double* mism;
   double* ws;
 };
-
-struct Blk {
-  double a, b, c, d;             // [[a, b], [c, d]]
-};
-
-__device__ __forceinline__ Blk ld_blk(const double* A, int64_t C, int p) {
-  const double* r = A + (int64_t)4 * p * C;
-  return {r[0], r[C], r[2 * C], r[3 * C]};
-}
-__device__ __forceinline__ void st_blk(double* A, int64_t C, int p, const Blk& x) {
-  double* r = A + (int64_t)4 * p * C;
-  r[0] = x.a;
-  r[C] = x.b;
-  r[2 * C] = x.c;
-  r[3 * C] = x.d;
-}
-__device__ __forceinline__ Blk mul(const Blk& x, const Blk& y) {
-  return {x.a * y.a + x.b * y.c, x.a * y.b + x.b * y.d, x.c * y.a + x.d * y.c, x.c * y.b + x.d * y.d};
-}
 
 // S_calc of bus i (MVA): U_i conj(sum_j Y_ij U_j) with U = e + j f
 __device__ __forceinline__ void bus_power(const dss2_pf_topology_t& t, const double* e, const double* f, int64_t C, int i, double& P,
@@ -136,60 +118,14 @@ __global__ void __launch_bounds__(PF_THREADS) k_pf_newton(PfArgs a) {
         st_blk(A, C, p, J);
       }
     }
-    // block LU, row by row: L[k,m] = A[k,m] inv(A[m,m]) for m < k ascending, A[k,j] -= L[k,m] A[m,j] (j > m); then invert A[k,k]
-    bool singular = false;
-    for (int k = 0; k < n && !singular; ++k) {
-      const int dk = __ldg(t.diag + k);
-      for (int p = __ldg(t.blk_ptr + k); p < dk; ++p) {
-        const Blk L = mul(ld_blk(A, C, p), ld_blk(A, C, __ldg(t.diag + __ldg(t.blk_col + p))));
-        st_blk(A, C, p, L);
-        for (int u = __ldg(t.upd_ptr + p); u < __ldg(t.upd_ptr + p + 1); ++u) {
-          const int dst = __ldg(t.upd + 2 * u), src = __ldg(t.upd + 2 * u + 1);
-          const Blk x = ld_blk(A, C, dst), y = mul(L, ld_blk(A, C, src));
-          st_blk(A, C, dst, {x.a - y.a, x.b - y.b, x.c - y.c, x.d - y.d});
-        }
-      }
-      const Blk D = ld_blk(A, C, dk);
-      const double det = D.a * D.d - D.b * D.c;
-      if (!(fabs(det) > 1e-12 * (fabs(D.a * D.d) + fabs(D.b * D.c)))) {
-        singular = true;
-        break;
-      }
-      const double r = 1.0 / det;
-      st_blk(A, C, dk, {D.d * r, -D.b * r, -D.c * r, D.a * r});
-    }
-    if (singular) break;
-    // forward: y_k = F_k - sum_{m<k} L[k,m] y_m
-    for (int k = 0; k < n; ++k) {
-      double yp = F[k * C], yq = F[(n + k) * C];
-      for (int p = __ldg(t.blk_ptr + k); p < __ldg(t.diag + k); ++p) {
-        const Blk L = ld_blk(A, C, p);
-        const int m = __ldg(t.blk_col + p);
-        const double xp = F[m * C], xq = F[(n + m) * C];
-        yp -= L.a * xp + L.b * xq;
-        yq -= L.c * xp + L.d * xq;
-      }
-      F[k * C] = yp;
-      F[(n + k) * C] = yq;
-    }
-    // back: x_k = inv(A[k,k]) (y_k - sum_{j>k} A[k,j] x_j), then the update (th, V) -= x
+    // block LU (block_lu.cuh), forward / back substitution, then the update (th, V) -= x
+    const BlockLu lu = {n, t.blk_ptr, t.blk_col, t.diag, t.upd_ptr, t.upd};
+    if (!block_lu_factor(lu, A, C)) break;
+    block_lu_solve(lu, A, F, C);
     for (int k = n - 1; k >= 0; --k) {
-      const int dk = __ldg(t.diag + k);
-      double yp = F[k * C], yq = F[(n + k) * C];
-      for (int p = dk + 1; p < __ldg(t.blk_ptr + k + 1); ++p) {
-        const Blk U = ld_blk(A, C, p);
-        const int j = __ldg(t.blk_col + p);
-        const double xp = F[j * C], xq = F[(n + j) * C];
-        yp -= U.a * xp + U.b * xq;
-        yq -= U.c * xp + U.d * xq;
-      }
-      const Blk D = ld_blk(A, C, dk);
-      const double xp = D.a * yp + D.b * yq, xq = D.c * yp + D.d * yq;
-      F[k * C] = xp;
-      F[(n + k) * C] = xq;
       const int i = __ldg(t.bus + k);
-      th[i * C] -= xp;
-      V[i * C] -= xq;
+      th[i * C] -= F[k * C];
+      V[i * C] -= F[(n + k) * C];
     }
   }
   // the state, and the slack injection in the load-positive convention

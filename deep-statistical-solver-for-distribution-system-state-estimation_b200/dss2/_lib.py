@@ -56,10 +56,22 @@ class PfTopology(Structure):
     ]
 
 
+class SeTopology(Structure):
+    """Mirror of `dss2_se_topology_t` (one state-estimation topology, dss2.estimation)."""
+    _fields_ = [
+        ("num_buses", c_int32), ("num_edges", c_int32), ("slack", c_int32), ("num_blocks", c_int32), ("num_updates", c_int32),
+        ("num_pairs", c_int32), ("max_support", c_int32),
+        ("edge_ft", c_void_p), ("inc_ptr", c_void_p), ("inc", c_void_p), ("sup_ptr", c_void_p), ("sup_pos", c_void_p),
+        ("pair_ptr", c_void_p), ("pair_blk", c_void_p), ("edge_blk", c_void_p), ("bus", c_void_p), ("blk_ptr", c_void_p),
+        ("blk_col", c_void_p), ("diag", c_void_p), ("upd_ptr", c_void_p), ("upd", c_void_p),
+    ]
+
+
 _P = c_void_p
 _G = POINTER(GraphStruct)
 _D = POINTER(AttnDrop)
 _T = POINTER(PfTopology)
+_ST = POINTER(SeTopology)
 _SIGNATURES = {
     "dss2_last_error": (c_char_p, []),
     "dss2_version": (c_int, []),
@@ -104,6 +116,9 @@ _SIGNATURES = {
     "dss2_powerflow_workspace_bytes": (c_size_t, [_T, c_int64]),
     "dss2_powerflow": (c_int, [_T, c_int64, _P, _P, _P, ctypes.c_double, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t,
                                c_int64, _P]),
+    "dss2_wls_estimate_workspace_bytes": (c_size_t, [_ST, c_int64]),
+    "dss2_wls_estimate": (c_int, [_ST, c_int64, _P, c_int64, _P, c_int64, _P, ctypes.c_double, ctypes.c_double, ctypes.c_double,
+                                  ctypes.c_double, c_int, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t, c_int64, _P]),
     "dss2_pflow": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, _P, _P]),
     "dss2_pflow_ex": (c_int, [_P, c_int64, _P, c_int64, _P, c_int64, _P, c_int, _P, _P]),
     "dss2_pflow_bwd": (c_int, [_G, _P, c_int64, _P, c_int64, _P, c_int, _P, _P, _P]),

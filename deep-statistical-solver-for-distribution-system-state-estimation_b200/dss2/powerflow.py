@@ -56,12 +56,33 @@ def symbolic(grid):
     y_gb = np.array([[ydict[k].real, ydict[k].imag] for k in keys], dtype=np.float64) * v_lv ** 2
     y_index = {k: i for i, k in enumerate(keys)}
 
-    # elimination order on the PQ graph: minimum degree (degree-0/1 buses, the leaves, come first), ties by bus id
+    # elimination order on the PQ graph (the slack is not in the reduced system)
     adj = [set() for _ in range(N)]
     for (i, j) in keys:
         if i != j and i != slack and j != slack:
             adj[i].add(j)
-    heap = [(len(adj[i]), i) for i in range(N) if i != slack]
+    el = block_elimination(adj, [i for i in range(N) if i != slack])
+    bus, rows = el["bus"], el["rows"]
+    blk_y = np.array([y_index.get((int(bus[k]), int(bus[c])), -1) for k, r in enumerate(rows) for c in r], dtype=np.int32)
+    blk_ptr, blk_col, diag, upd_ptr, upd, fill, pos = (el[k] for k in ("blk_ptr", "blk_col", "diag", "upd_ptr", "upd", "fill", "pos"))
+    return {"num_buses": N, "slack": slack, "v_lv": v_lv, "closed": np.nonzero(closed)[0], "edge_ft": np.stack([frm, to], 1).astype(np.int32),
+            "edge_gb": np.ascontiguousarray(ce[:, 2:6]), "y_ptr": y_ptr, "y_col": y_col, "y_gb": y_gb, "bus": bus, "pos": pos,
+            "blk_ptr": blk_ptr, "blk_col": blk_col, "blk_y": blk_y, "diag": diag, "upd_ptr": upd_ptr, "upd": upd, "fill": fill}
+
+
+def block_elimination(adj, nodes):
+    """Minimum-degree elimination of the graph `adj` (list of neighbour sets indexed by bus; consumed) restricted to `nodes`, and the
+    2x2-block pattern with fill and the update lists of the row-wise block LU in csrc/block_lu.cuh.  Buses of degree 0/1 (the leaves)
+    come first, ties by bus id.  Returns a dict:
+      bus[k]            bus eliminated at position k; pos[i] its inverse (-1 off `nodes`)
+      rows[k]           columns of block row k, ascending (host lists)
+      blk_ptr/blk_col   CSR of the factor's block pattern in position order, columns ascending
+      diag[k]           block (k, k); where[k][m] the block (k, m) (host dicts)
+      upd_ptr/upd       per lower block p = (k, m): the pairs (block (k, j), block (m, j)) over the upper entries j > m of row m,
+                        i.e. A[k, j] -= L[k, m] A[m, j]
+      fill              number of fill pairs (blocks off the graph, counted once per bus pair)"""
+    N = len(adj)
+    heap = [(len(adj[i]), i) for i in nodes]
     heapq.heapify(heap)
     done = np.zeros(N, dtype=bool)
     order, upper, fill = [], {}, 0
@@ -83,7 +104,7 @@ def symbolic(grid):
                     fill += 1
         for a in nb:
             heapq.heappush(heap, (len(adj[a]), a))
-    n = N - 1
+    n = len(order)
     bus = np.array(order, dtype=np.int32)
     pos = np.full(N, -1, dtype=np.int64)
     pos[bus] = np.arange(n)
@@ -100,7 +121,6 @@ def symbolic(grid):
     blk_ptr[1:] = np.cumsum([len(r) for r in rows])
     blk_col = np.array([c for r in rows for c in r], dtype=np.int32)
     where = [{c: int(blk_ptr[k]) + i for i, c in enumerate(r)} for k, r in enumerate(rows)]
-    blk_y = np.array([y_index.get((int(bus[k]), int(bus[c])), -1) for k, r in enumerate(rows) for c in r], dtype=np.int32)
     diag = np.array([where[k][k] for k in range(n)], dtype=np.int32)
     upd_ptr = np.zeros(blk_col.size + 1, dtype=np.int32)
     upd = []
@@ -111,9 +131,8 @@ def symbolic(grid):
                 upd.extend((where[k][j], where[m][j]) for j in rows[m] if j > m)
             upd_ptr[p + 1] = len(upd)
     upd = np.array(upd, dtype=np.int32).reshape(-1, 2)
-    return {"num_buses": N, "slack": slack, "v_lv": v_lv, "closed": np.nonzero(closed)[0], "edge_ft": np.stack([frm, to], 1).astype(np.int32),
-            "edge_gb": np.ascontiguousarray(ce[:, 2:6]), "y_ptr": y_ptr, "y_col": y_col, "y_gb": y_gb, "bus": bus, "pos": pos,
-            "blk_ptr": blk_ptr, "blk_col": blk_col, "blk_y": blk_y, "diag": diag, "upd_ptr": upd_ptr, "upd": upd, "fill": fill}
+    return {"bus": bus, "pos": pos, "rows": rows, "where": where, "blk_ptr": blk_ptr, "blk_col": blk_col, "diag": diag,
+            "upd_ptr": upd_ptr, "upd": upd, "fill": fill}
 
 
 _CACHE = {}

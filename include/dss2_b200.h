@@ -362,6 +362,66 @@ int dss2_powerflow(const dss2_pf_topology_t* topo, int64_t S, const double* p_mw
                    double* q_from, double* p_to, double* q_to, int32_t* iterations, uint8_t* converged, double* max_mismatch,
                    void* workspace, size_t workspace_bytes, int64_t chunk, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Classical weighted-least-squares state estimation, batched: the estimator the reference compares DSS2 against
+ * (case_study.py:1226-1357, pandapower's WLS estimator) on the measurements of the physics-informed loss (data.py:393-459).
+ * Per scenario of N buses and E closed edges, with Z, R, Z', R' the de-normalised, masked measurements and weights of the loss
+ * (data.py:397-409; a normalised value of exactly 0 is absent), fp64 on the fp32 inputs promoted exactly:
+ *   J_s(V, th) = w_v sum_n [R_n0 (Z_n0 - V_n)^2 + R_n1 (Z_n1 - th_n)^2] + w_p sum_n [R_n2 (Z_n2 - p_n)^2 + R_n3 (Z_n3 - q_n)^2]
+ *              + w_pf sum_e [R'_e0 (Z'_e0 - P_f,e)^2 + R'_e1 (Z'_e1 - Q_f,e)^2]
+ * th_slack = 0 (x column 9, data.py:412-413); p_n = -sum_{to=n} P_t - sum_{from=n} P_f and the same for q (data.py:428-429); the
+ * flows of the pi-model (data.py:370-376, phase shift ignored) with c = V_lv^2, V_lv = min vn_kv (x column 8) of the scenario, and
+ * G, B, Gs, Bs from edge_attr columns 6-9.  Classical WLS: w_v = w_p = w_pf = 1; the loss's data term: lam_v / N, lam_p / N, lam_pf / E.
+ * Gauss-Newton over the 2N - 1 unknowns (th, V) from a flat start (V = 1, th = 0): the gain matrix H^T W H as 2x2 (th, V) blocks per
+ * pair of buses that share a measurement, the slack's block with identity in its th row and column, factorised by the block LU of
+ * the power flow in the host's elimination order, in double-double (a weight near 1e12 makes the fp64 Schur complements cancel).
+ * The step is halved until J_s does not grow (beyond 1e-12 relative), which keeps Gauss-Newton from diverging on scenarios with
+ * large residuals.  Stops when the full step max |dx| <= tol (converged), after max_iter updates, or when no halving (down to
+ * 2^-39) decreases J_s.
+ * Topology (built once on the host, dss2.estimation.symbolic; every array DEVICE, int32; "position" = elimination position):
+ *   edge_ft [E,2]: local (from, to) of the closed edges, the batch's edge order;
+ *   inc_ptr [N+1], inc [.,3]: per bus its incident edges as (edge, end 0 = from / 1 = to, support slot of the other end);
+ *   sup_ptr [N+1], sup_pos: per bus the positions of its support {i} u nbr(i), slot 0 = the bus itself;
+ *   pair_ptr [N+1], pair_blk: per bus the block of every (slot a, slot b) of its support, row-major over (a, b);
+ *   edge_blk [E,4]: blocks (ii, ij, ji, jj) of every edge; bus [N]: bus at each position;
+ *   blk_ptr, blk_col, diag, upd_ptr, upd: the block pattern with fill and the LU's update lists (as dss2_pf_topology_t).
+ * dss2_wls_estimate: B scenarios of one topology in PyG order: x [B N, >= 11] (row stride x_stride), edge_attr [B E, >= 13],
+ * stats28 = x_mean[8], x_std[8], edge_mean[6], edge_std[6] (fp32, device).  Out: vm_pu, va_rad [B N] f64, output [B N, 2] f32 =
+ * ((V - x_mean0) / x_std0, th) (the model's output convention), objective [B] = J_s at the returned state, iterations [B] = updates
+ * applied, converged [B] u8, max_step [B] = the last full step max |dx|.  A pivot with |det| <= 1e-12 (|ad| + |bc|), a
+ * non-finite value, max_iter updates without convergence or a step without descent give converged = 0 for that scenario only.
+ * Scenarios run `chunk` per launch, one thread each, in `workspace` (dss2_wls_estimate_workspace_bytes(topo, chunk) = 8 chunk
+ * (16 N + 28 E + 8 blocks + 4 max_support) bytes, index-major, the blocks and the right-hand side in double-double); no atomics, so a scenario's result does not depend on the chunk or the other scenarios.  No host synchronisation, no allocation.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dss2_se_topology {
+  int32_t num_buses;        /* N */
+  int32_t num_edges;        /* E */
+  int32_t slack;
+  int32_t num_blocks;
+  int32_t num_updates;
+  int32_t num_pairs;        /* sum over buses of |support|^2 */
+  int32_t max_support;
+  const int32_t* edge_ft;
+  const int32_t* inc_ptr;
+  const int32_t* inc;
+  const int32_t* sup_ptr;
+  const int32_t* sup_pos;
+  const int32_t* pair_ptr;
+  const int32_t* pair_blk;
+  const int32_t* edge_blk;
+  const int32_t* bus;
+  const int32_t* blk_ptr;
+  const int32_t* blk_col;
+  const int32_t* diag;
+  const int32_t* upd_ptr;
+  const int32_t* upd;
+} dss2_se_topology_t;
+size_t dss2_wls_estimate_workspace_bytes(const dss2_se_topology_t* topo, int64_t chunk);
+int dss2_wls_estimate(const dss2_se_topology_t* topo, int64_t B, const float* x, int64_t x_stride, const float* edge_attr,
+                      int64_t ea_stride, const float* stats28, double w_v, double w_p, double w_pf, double tol, int max_iter,
+                      double* vm_pu, double* va_rad, float* output, double* objective, int32_t* iterations, uint8_t* converged,
+                      double* max_step, void* workspace, size_t workspace_bytes, int64_t chunk, void* stream);
+
 /* Validation metrics of one batch (SURVEY.md 8f-4, dss2_run.py:183-209) in one kernel: x [Nt,>=11] (column 9 = slack flag),
  * edge_attr [Et,>=13] (columns 6.. = branch parameters), output [Nt,2] = model output (normalised V, raw theta), y [Nt,2] = labels.
  * sums19 (device, fp64): [0..3] sum (dV)^2, |dV|, (dth)^2, |dth| with V = out0*x_std0 + x_mean0 and th = out1*(1-slack);
